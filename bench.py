@@ -10,8 +10,12 @@ the export interpolation over that batch. With N GPUs the SAME batch is sharded 
 (`parallel.snapshot_window`: rank r interpolates T/N snapshots of all cells) -- strong scaling; the sampled grid and
 the KNN tables are computed on rank 0 and broadcast over NCCL once, there is no collective inside the step.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl s3b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl s3b200|reference] [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...                     (one rank per GPU)
+
+`--dump-outputs DIR` writes what the last timed step computed as DIR/p.npy [n, 1, T] and DIR/U.npy [n, 2, T] (float32)
+for a fixed, seeded sample of n grid cells (at most 64 MB in all). The inputs are seeded, so two builds of the project
+can be compared output for output.
 
 `--impl reference` times the reference's own CPU `interpolate_data` (unmodified, from oracle/_ref; the oracle port if
 that install is missing) with all host threads on the same workload.
@@ -22,6 +26,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -41,6 +46,7 @@ N_POINTS, N_SNAP = synth.CONFIGS["C2"][0], synth.CONFIGS["C2"][1]
 GRID_KW = dict(uniform_level=5, min_metric=0.75)
 K_NEIGHBORS = 8
 L2_BYTES = 126e6
+DUMP_BYTES = 64 * 10**6
 
 
 def geometries(geo):
@@ -277,7 +283,7 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ our arm
-def run_ours(args):
+def run_ours(args, tmp_dir):
     import torch.distributed as dist
     import sparsespatialsampling_b200 as s3
     from sparsespatialsampling_b200 import _lib
@@ -327,7 +333,7 @@ def run_ours(args):
         # the second is the steady-state number reported as grid_gen_s; both produce the same grid
         for attempt in range(2):
             t0 = time.time()
-            sc = s3.SparseSpatialSampling(x, metric, geometries(s3.geometry), "/tmp/s3b200_bench", "c2", **{
+            sc = s3.SparseSpatialSampling(x, metric, geometries(s3.geometry), tmp_dir, "c2", **{
                 "uniform_levels": GRID_KW["uniform_level"], "min_metric": GRID_KW["min_metric"]})
             sc.execute_grid_generation()
             pt.cuda.synchronize()
@@ -416,8 +422,14 @@ def run_ours(args):
     # `value_incl_table_broadcast` charged in full to these K steps.
     value = units_step / (ms_step * 1e-3)
     value_incl_bcast = units_step * args.steps / ((ms_total + bcast_ms) * 1e-3)
-    out_p, out_u = sets[0][2], sets[0][3]
+    out_p, out_u = sets[(args.steps - 1) % len(sets)][2:]          # the results of the last timed step
     check_p, check_u = out_p.clone(), out_u.clone()
+    if args.dump_outputs:
+        n_dump = min(n_cells, (DUMP_BYTES - 4096) // (3 * ts * 4))     # 4096: room for the two .npy headers
+        rows = pt.from_numpy(np.sort(np.random.default_rng(0).choice(n_cells, n_dump, replace=False))).to(dev)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "p.npy"), out_p[rows].cpu().numpy())
+        np.save(os.path.join(args.dump_outputs, "U.npy"), out_u[rows].cpu().numpy())
 
     aux_steps = max(10, min(args.steps, 50))
     dense_sets = make_sets(False, pt.float32)
@@ -437,7 +449,7 @@ def run_ours(args):
     g = _Grid()
     g.n_dimensions, g.faces, g.vertices, g.levels = 2, None, None, None
     g.centers, g.metric, g.size_initial_cell = centers, metric, 2.2
-    g.save_path, g.save_name, g.grid_name = "/tmp/s3b200_bench", f"c2_rank{rank}", "grid"
+    g.save_path, g.save_name, g.grid_name = tmp_dir, f"c2_rank{rank}", "grid"
 
     def e2e_run(async_host):
         exp = ExportData(g, write_times=[str(i) for i in range(N_SNAP)], write_files=False, device=dev,
@@ -609,11 +621,19 @@ def main():
     ap.add_argument("--no-svd", action="store_true", help="skip the SVD stage report")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--full", action="store_true", help="reference arm: all snapshots per step whatever it takes")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results (a seeded sample of cells) as DIR/p.npy and DIR/U.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl s3b200 in a single process")
     if args.impl == "reference":
         run_reference(args)
     else:
-        run_ours(args)
+        # grid files written by the grid generation go to a directory of this run, removed at the end
+        with tempfile.TemporaryDirectory(prefix="s3b200_bench_") as tmp_dir:
+            run_ours(args, tmp_dir)
 
 
 if __name__ == "__main__":

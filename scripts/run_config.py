@@ -17,6 +17,7 @@ import argparse
 import json
 import os
 import sys
+import tempfile
 import time
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -40,7 +41,8 @@ def fill_field(out: pt.Tensor, coords: pt.Tensor, n_total: int, comps: int, xc: 
     return out
 
 
-def config(name: str, n_cells_max, stl_subdiv: int = 4):
+def config(name: str, n_cells_max, stl_subdiv: int = 4, tmp_dir: str = None):
+    """Cloud, geometries, wake centre and grid options of a configuration; C5 writes its STL body into ``tmp_dir``."""
     geo = s3.geometry
     if name == "C3":
         x = synth.airfoil2d_cloud(synth.CONFIGS["C3"][0], seed=0)
@@ -58,7 +60,7 @@ def config(name: str, n_cells_max, stl_subdiv: int = 4):
         from tests.stl_util import icosphere_triangles, write_binary_stl
         x = synth.cylinder3d_cloud(synth.CONFIGS["C5"][0], seed=0)
         zmax = synth.CYL3D["upper"][2]
-        stl = "/tmp/s3b200_c5_body.stl"
+        stl = os.path.join(tmp_dir, "c5_body.stl")
         write_binary_stl(stl, icosphere_triangles(stl_subdiv, 0.12, (0.8, 1.0, zmax / 2)))
         geoms = [geo.CubeGeometry("domain", True, synth.CYL3D["lower"], synth.CYL3D["upper"]),
                  geo.GeometrySTL3D("body", False, stl, refine=True)]
@@ -66,7 +68,7 @@ def config(name: str, n_cells_max, stl_subdiv: int = 4):
     raise SystemExit(f"unknown config {name}")
 
 
-def main():
+def main(tmp_dir: str):
     ap = argparse.ArgumentParser()
     ap.add_argument("name", choices=["C3", "C4", "C5"])
     ap.add_argument("--svd", action="store_true", help="weighted SVD of the exported matrix (always on for C5)")
@@ -88,7 +90,7 @@ def main():
         for kv in args.tune.split(","):
             key, val = kv.split("=")
             _lib.tune(int(key), int(val))
-    x, geoms, wake, grid_kw = config(args.name, args.n_cells_max, args.stl_subdiv)
+    x, geoms, wake, grid_kw = config(args.name, args.n_cells_max, args.stl_subdiv, tmp_dir)
     d = x.size(1)
     k = 8 if d == 2 else 26
     T = args.snapshots or synth.CONFIGS[args.name][1]
@@ -97,7 +99,7 @@ def main():
 
     # ---- grid generation
     t0 = time.time()
-    sc = s3.SparseSpatialSampling(x, metric, geoms, "/tmp/s3b200_cfg", args.name.lower(), **grid_kw,
+    sc = s3.SparseSpatialSampling(x, metric, geoms, tmp_dir, args.name.lower(), **grid_kw,
                                   exact_topology=not args.lattice_vertices)
     t_setup = time.time() - t0
     sc.execute_grid_generation()
@@ -275,4 +277,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    # the STL body and the grid files are written to a directory of this run, removed at the end
+    with tempfile.TemporaryDirectory(prefix="s3b200_cfg_") as tmp:
+        main(tmp)

@@ -98,12 +98,16 @@ def _worker(rank, world, port, tmp):
         dist.destroy_process_group()
 
 
-def test_sharded_export_world_size_2_equals_single_process(tmp_path):
+def test_sharded_export_world_size_2_equals_single_process(tmp_path, monkeypatch):
     """ExportData(distributed=True) under gloo: table broadcast, snapshot windows, per-rank part files, one XDMF and the
     Dataloader that follows the part list -- against the same export done by one process."""
+    from sparsespatialsampling_b200 import _lib, export
     from sparsespatialsampling_b200.data import Dataloader
     world = 2
     mp.spawn(_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
+    # the single-process run happens in this process: the CPU stand-ins _worker installs must not outlive this test
+    monkeypatch.setattr(_lib, "require_cuda", _lib.require_cuda)
+    monkeypatch.setattr(export, "interp_gather", export.interp_gather)
     _worker(0, 1, 0, str(tmp_path))                                   # single process, same code
     assert sorted(os.listdir(tmp_path))[:3] == ["sharded.h5", "sharded.part1.h5", "sharded.xdmf"]
     many, one = Dataloader(str(tmp_path), "sharded.h5"), Dataloader(str(tmp_path / "single"), "sharded.h5")
