@@ -38,9 +38,11 @@ static int g_kunroll = 0;          // key 7: neighbour-loop unroll (row loads in
 static int g_persistent = -1;      // key 8: part-warp persistent kernel: -1 = short rows (see launch_interp), 0 = never, 1 = whenever possible
 static int g_lanes_per_cell = 0;   // key 13: lanes per cell of that kernel (16 or 32), 0 = by row length
 static int g_persist_ctas = 0;     // key 12: resident CTAs per SM it is compiled for (3: 80 registers, 4: 64), 0 = by row length
+static int g_persist_cap = 0;      // key 15: at most this many CTAs of that kernel (tests: several sweeps at small sizes), 0 = no cap
 extern int g_tc_seg_kblocks;
 extern int g_tc_flush_segments;
 extern int g_tc_pair;
+extern int g_plane_rows_cap;       // key 17 (csrc/svd.cu): rows per TF32 plane chunk of the Gram / projection kernels, 0 = no cap
 extern int g_curve;          // csrc/knn.cu: 0 = Morton, 1 = Hilbert order of the KNN index and of the processing order (key 30)
 
 template <typename T, int V>
@@ -434,7 +436,8 @@ static int launch_interp(const void* data, const int32_t* idx, const void* w, in
             if (slot) *slot = resident;                                                                            \
         }                                                                                                          \
         const int64_t want = ceil_div(n_cells, (int64_t)pw * sub);                                                 \
-        const int64_t ctas = want < (int64_t)resident ? want : (int64_t)resident;                                  \
+        int64_t ctas = want < (int64_t)resident ? want : (int64_t)resident;                                        \
+        if (g_persist_cap > 0 && ctas > g_persist_cap) ctas = g_persist_cap;                                       \
         kern<<<(unsigned)ctas, threads, sm, stream>>>(d_f, idx, w_f, n_cells, k, out_row, o_f, g, n_comp, store_w); \
     } while (0)
 #define S3_PARTWARP_C(L, K_, R) do { if (ku == 8) S3_PARTWARP(L, 8, R, 2); else if (per_sm_built == 4) S3_PARTWARP(L, 4, R, 4); else S3_PARTWARP(L, 4, R, 3); } while (0)
@@ -524,7 +527,7 @@ static int launch_interp(const void* data, const int32_t* idx, const void* w, in
 using namespace s3;
 
 // A/B harness hook (scripts/, tests of the variants): NOT declared in include/s3b200.h. Keys: see the knobs above;
-// 10 / 11 / 14 belong to the tensor-core Gram kernel (csrc/svd.cu).
+// 10 / 11 / 14 / 17 belong to the tensor-core Gram and projection kernels (csrc/svd.cu).
 extern "C" int s3x_tune(int key, int value) {
     switch (key) {
         case 1: S3_REQUIRE(value >= 1 && value <= 16, "s3x_tune: warps per CTA must be 1..16"); g_warps_per_cta = value; return S3_OK;
@@ -538,11 +541,13 @@ extern "C" int s3x_tune(int key, int value) {
         case 7: S3_REQUIRE(value == 0 || value == 1 || value == 4 || value == 8, "s3x_tune: neighbour-loop unroll must be 0 (auto), 1, 4 or 8"); g_kunroll = value; return S3_OK;
         case 8: S3_REQUIRE(value >= -1 && value <= 1, "s3x_tune: part-warp kernel must be -1 (short rows), 0 (never) or 1 (whenever possible)"); g_persistent = value; return S3_OK;
         case 12: S3_REQUIRE(value == 0 || value == 3 || value == 4, "s3x_tune: resident CTAs per SM must be 0 (by row length), 3 or 4"); g_persist_ctas = value; return S3_OK;
+        case 15: S3_REQUIRE(value >= 0 && value <= (1 << 20), "s3x_tune: part-warp CTA cap must be 0 (none) or >= 1"); g_persist_cap = value; return S3_OK;
         case 13: S3_REQUIRE(value == 0 || value == 16 || value == 32, "s3x_tune: lanes per cell must be 0 (by row length), 16 or 32"); g_lanes_per_cell = value; return S3_OK;
         case 30: S3_REQUIRE(value == 0 || value == 1, "s3x_tune: curve must be 0 (Morton) or 1 (Hilbert)"); g_curve = value; return S3_OK;
         case 10: S3_REQUIRE(value >= 1 && value <= (1 << 20), "s3x_tune: K-blocks per TMEM segment must be >= 1"); g_tc_seg_kblocks = value; return S3_OK;
         case 11: S3_REQUIRE(value >= 1 && value <= (1 << 20), "s3x_tune: segments per fp64 flush must be >= 1"); g_tc_flush_segments = value; return S3_OK;
         case 14: S3_REQUIRE(value == 0 || value == 1, "s3x_tune: paired Gram kernel must be 0 or 1"); g_tc_pair = value; return S3_OK;
+        case 17: S3_REQUIRE(value >= 0, "s3x_tune: plane-row cap must be 0 (none) or >= 1"); g_plane_rows_cap = value; return S3_OK;
     }
     s3::set_error("s3x_tune: unknown key %d", key);
     return S3_ERR_INVALID;

@@ -46,17 +46,20 @@ row_mean_kernel(const float* __restrict__ a, int64_t m, int64_t t, float* __rest
 constexpr int kGT = 128;     // output tile (kGT x kGT) per CTA
 constexpr int kGK = 16;      // rows of A per shared-memory step
 constexpr int kGThreads = 256;
+// rows of A per K-split at most: a split sums its rows in fp32 before the fp64 reduce, and that error grows with its
+// length (600 000 x 2000 in 5 splits of 120 000 rows: 5.8e-5 of sqrt(G_ii G_jj) on a B200, against 2e-5 as the bound)
+constexpr int64_t kGSplitRows = 8192;
 
 __global__ void __launch_bounds__(kGThreads)
 gram_kernel(const float* __restrict__ a, const float* __restrict__ mean, const float* __restrict__ vol, int vol_div,
-            int64_t m, int64_t t, int tiles, int64_t rows_per_split, float* __restrict__ partial) {
+            int64_t row0, int64_t m, int64_t t, int tiles, int64_t rows_per_split, float* __restrict__ partial) {
     __shared__ float sa[kGK][kGT];
     __shared__ float sb[kGK][kGT];
     // upper-triangular tile pair (ti <= tj) from the linear tile id
     int tid_lin = blockIdx.x, ti = 0;
     while (tid_lin >= tiles - ti) { tid_lin -= tiles - ti; ++ti; }
     const int tj = ti + tid_lin;
-    const int64_t r0 = (int64_t)blockIdx.y * rows_per_split;
+    const int64_t r0 = row0 + (int64_t)blockIdx.y * rows_per_split;
     const int64_t r1 = (r0 + rows_per_split) < m ? (r0 + rows_per_split) : m;
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;     // 16 x 16 threads, 8 x 8 outputs each
     float acc[8][8];
@@ -108,16 +111,16 @@ gram_kernel(const float* __restrict__ a, const float* __restrict__ mean, const f
     }
 }
 
-// sum the K-splits in fp64 and mirror the upper triangle
+// sum the K-splits in fp64 (and add to g: accumulate) and mirror the upper triangle
 __global__ void __launch_bounds__(256)
-gram_reduce_kernel(const float* __restrict__ partial, int splits, int64_t t, double* __restrict__ g) {
+gram_reduce_kernel(const float* __restrict__ partial, int splits, int64_t t, int accumulate, double* __restrict__ g) {
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= t * t) return;
     const int64_t i = e / t, j = e % t;
     const int64_t ti = i / kGT, tj = j / kGT;
     // tiles with ti <= tj were computed; take (i,j) from there, or its transpose
     const int64_t src = (ti <= tj) ? (i * t + j) : (j * t + i);
-    double acc = 0.0;
+    double acc = accumulate ? g[e] : 0.0;
     for (int s = 0; s < splits; ++s) acc += (double)partial[(int64_t)s * t * t + src];
     g[e] = acc;
 }
@@ -195,6 +198,8 @@ constexpr size_t kTcSmemBytes = (size_t)kTcStages * kTcStageBytes + 1024;
 int g_tc_seg_kblocks = 8;      // K-blocks accumulated in TMEM before the epilogue takes over (s3_set_tuning key 10)
 int g_tc_pair = 1;             // clusters of two CTAs sharing B via TMA multicast (s3_set_tuning key 14)
 int g_tc_flush_segments = 128;  // TMEM segments summed in fp32 registers per fp64 flush (s3_set_tuning key 11)
+int g_plane_rows_cap = 0;       // rows per plane chunk of gram_tc / project_tc at most (key 17; tests reach the chunked
+                                // accumulation at small sizes), 0 = planes of up to 2 GB
 
 // Centre, scale and split the rows [row0, row0 + n_rows) of A into TF32 planes, layout [n_groups][plane_rows][32]:
 //   b = (a - mean) * sqrt(vol);  hi = tf32_rna(b);  lo = b - hi  (exact in fp32; the tensor core drops lo's low bits).
@@ -586,6 +591,10 @@ constexpr int kPjBM = 128;
 constexpr int kPjStages = 2;
 constexpr int kPjThreads = 6 * 32;
 constexpr int kPjABytes = kPjBM * 128;                       // one plane tile: 128 rows x 32 floats
+// 32-column groups per TMEM segment at most (3xTF32: 384 MMAs, the chain length of T = 2000 at r = 256); longer t ranges
+// run as several launches that add into U. One launch with two segments of 128 / 256 groups (r = 256, T = 8192 / 16 384)
+// measured 3.2e-5 / 5.1e-5 of the largest entry on a B200, split launches 7e-6 (tests/test_svd_scale_gpu.py).
+constexpr int kPjSegGroups = 32;
 
 __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
     asm volatile(
@@ -627,9 +636,9 @@ project_prepare_w_kernel(const float* __restrict__ vs, int64_t t, int r, int col
 
 __global__ void __launch_bounds__(kPjThreads, 1)
 project_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo,
-                  const __grid_constant__ CUtensorMap map_whi, const __grid_constant__ CUtensorMap map_wlo, int n_groups,
-                  int r_pad, int tmem_cols, int n_seg, int passes, const float* __restrict__ vol, int vol_div, int64_t row0,
-                  int64_t m, int r, int col0, float* __restrict__ u) {
+                  const __grid_constant__ CUtensorMap map_whi, const __grid_constant__ CUtensorMap map_wlo, int g0,
+                  int n_groups, int r_pad, int tmem_cols, int n_seg, int passes, const float* __restrict__ vol, int vol_div,
+                  int64_t row0, int64_t m, int r, int col0, int add, float* __restrict__ u) {
     extern __shared__ __align__(1024) unsigned char pj_smem_raw[];
     __shared__ __align__(8) uint64_t full_bar[kPjStages];
     __shared__ __align__(8) uint64_t empty_bar[kPjStages];
@@ -672,11 +681,11 @@ project_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
                 if (round > 0) mbar_wait_wd(&empty_bar[s], (round - 1) & 1u);
                 unsigned char* st = ring_ptr + (size_t)s * stage_bytes;
                 mbar_expect_tx(&full_bar[s], tx);
-                tma_load_3d(st, &map_hi, 0, tile_row, g, &full_bar[s]);
-                tma_load_2d(st + 2 * kPjABytes, &map_whi, g * 32, 0, &full_bar[s]);
+                tma_load_3d(st, &map_hi, 0, tile_row, g0 + g, &full_bar[s]);
+                tma_load_2d(st + 2 * kPjABytes, &map_whi, (g0 + g) * 32, 0, &full_bar[s]);
                 if (passes == 3) {
-                    tma_load_3d(st + kPjABytes, &map_lo, 0, tile_row, g, &full_bar[s]);
-                    tma_load_2d(st + 2 * kPjABytes + w_bytes, &map_wlo, g * 32, 0, &full_bar[s]);
+                    tma_load_3d(st + kPjABytes, &map_lo, 0, tile_row, g0 + g, &full_bar[s]);
+                    tma_load_2d(st + 2 * kPjABytes + w_bytes, &map_wlo, (g0 + g) * 32, 0, &full_bar[s]);
                 }
             }
         }
@@ -739,7 +748,7 @@ project_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
                 float* o = u + row * r + col0 + c0;
 #pragma unroll
                 for (int c = 0; c < 32; ++c)
-                    if (col0 + c0 + c < r) o[c] = acc[c] * scale;
+                    if (col0 + c0 + c < r) o[c] = add ? __fadd_rn(o[c], acc[c] * scale) : acc[c] * scale;
             }
         }
     }
@@ -773,23 +782,31 @@ static int gram_simt(const float* d_a, const float* d_mean, const float* d_vol, 
                      double* d_gram, cudaStream_t st) {
     const int tiles = (int)ceil_div(t, kGT);
     const int n_pairs = tiles * (tiles + 1) / 2;
-    // enough K-splits to fill the GPU, bounded by the scratch they need
-    int splits = (int)ceil_div(4 * kNumSMs, n_pairs);
+    // enough K-splits to fill the GPU, of at most kGSplitRows rows each
+    int64_t splits = ceil_div(4 * kNumSMs, n_pairs);
     if (splits < 1) splits = 1;
     const int64_t max_splits_mem = (int64_t)(2ll << 30) / (t * t * 4);
-    if (splits > max_splits_mem) splits = (int)(max_splits_mem > 0 ? max_splits_mem : 1);
-    if ((int64_t)splits > ceil_div(m, kGK)) splits = (int)ceil_div(m, kGK);
+    if (splits > max_splits_mem) splits = max_splits_mem > 0 ? max_splits_mem : 1;
+    if (splits > ceil_div(m, kGK)) splits = ceil_div(m, kGK);
     int64_t rows_per_split = ceil_div(ceil_div(m, splits), kGK) * kGK;
-    splits = (int)ceil_div(m, rows_per_split);
+    if (rows_per_split > kGSplitRows) rows_per_split = kGSplitRows;
+    splits = ceil_div(m, rows_per_split);
+    // splits per launch, bounded by the scratch they need; later passes add into the fp64 result
+    int64_t per_pass = splits < max_splits_mem ? splits : (max_splits_mem > 0 ? max_splits_mem : 1);
+    if (per_pass > 65535) per_pass = 65535;
     Scratch scratch(st);
     float* partial = nullptr;
-    S3_TRY(scratch.alloc(&partial, (size_t)splits * t * t));
-    S3_CUDA(cudaMemsetAsync(partial, 0, sizeof(float) * (size_t)splits * t * t, st));
-    dim3 grid((unsigned)n_pairs, (unsigned)splits);
-    gram_kernel<<<grid, kGThreads, 0, st>>>(d_a, d_mean, d_vol, vol_div, m, t, tiles, rows_per_split, partial);
-    gram_reduce_kernel<<<(unsigned)ceil_div(t * t, 256), 256, 0, st>>>(partial, splits, t, d_gram);
-    S3_LAUNCH_CHECK();
-    note_launch(2);
+    S3_TRY(scratch.alloc(&partial, (size_t)per_pass * t * t));
+    S3_CUDA(cudaMemsetAsync(partial, 0, sizeof(float) * (size_t)per_pass * t * t, st));
+    for (int64_t s0 = 0; s0 < splits; s0 += per_pass) {
+        const int64_t n = (splits - s0) < per_pass ? (splits - s0) : per_pass;
+        dim3 grid((unsigned)n_pairs, (unsigned)n);
+        gram_kernel<<<grid, kGThreads, 0, st>>>(d_a, d_mean, d_vol, vol_div, s0 * rows_per_split, m, t, tiles,
+                                                rows_per_split, partial);
+        gram_reduce_kernel<<<(unsigned)ceil_div(t * t, 256), 256, 0, st>>>(partial, (int)n, t, s0 > 0, d_gram);
+        S3_LAUNCH_CHECK();
+        note_launch(2);
+    }
     return S3_OK;
 }
 
@@ -814,6 +831,7 @@ static int gram_tc(const float* d_a, const float* d_mean, const float* d_vol, in
     else for (int ti = 0; ti < n_i; ++ti) tiles += n_j - tc_first_tj(ti);
     // rows of A per chunk: each plane at most 2 GB
     int64_t plane_rows = ((int64_t)(1ll << 31) / (t_pad * 4)) & ~(int64_t)(kTcKB - 1);
+    if (g_plane_rows_cap > 0 && plane_rows > g_plane_rows_cap) plane_rows = g_plane_rows_cap & ~(int64_t)(kTcKB - 1);
     if (plane_rows < kTcKB) plane_rows = kTcKB;
     const int64_t m_pad = ceil_div(m, kTcKB) * kTcKB;
     if (plane_rows > m_pad) plane_rows = m_pad;
@@ -924,6 +942,7 @@ static int project_tc(const float* d_a, const float* d_mean, const float* d_vol,
     const int n_groups = (int)(t_pad / 32);
     // rows of A per chunk: each plane at most 2 GB, a multiple of the 128-row tile
     int64_t plane_rows = ((int64_t)(1ll << 31) / (t_pad * 4)) & ~(int64_t)(kPjBM - 1);
+    if (g_plane_rows_cap > 0 && plane_rows > g_plane_rows_cap) plane_rows = g_plane_rows_cap & ~(int64_t)(kPjBM - 1);
     if (plane_rows < kPjBM) plane_rows = kPjBM;
     const int64_t m_pad = ceil_div(m, (int64_t)kPjBM) * kPjBM;
     if (plane_rows > m_pad) plane_rows = m_pad;
@@ -960,6 +979,7 @@ static int project_tc(const float* d_a, const float* d_mean, const float* d_vol,
         const int tmem_cols = r_pad > 128 ? 512 : 256;
         int n_seg = tmem_cols / r_pad;
         if (n_seg > 8) n_seg = 8;
+        const int launch_groups = n_seg * kPjSegGroups;            // t range of one launch: segments of <= kPjSegGroups
         if (n_seg > n_groups) n_seg = n_groups;
         project_prepare_w_kernel<<<(unsigned)ceil_div((int64_t)r_pad * t_pad, (int64_t)256), 256, 0, st>>>(
             d_vs, t, r, col0, r_pad, t_pad, whi, wlo);
@@ -987,11 +1007,15 @@ static int project_tc(const float* d_a, const float* d_mean, const float* d_vol,
             const int64_t rows_pad = ceil_div(rows, (int64_t)kPjBM) * kPjBM;
             gram_prepare_kernel<<<(unsigned)ceil_div(rows_pad * 32, (int64_t)256), 256, 0, st>>>(
                 d_a, d_mean, d_vol, vol_div, row0, rows_pad, m, t, n_groups, plane_rows, hi, lo);
-            project_tc_kernel<<<(unsigned)(rows_pad / kPjBM), kPjThreads, smem, st>>>(
-                map_hi, map_lo, map_whi, map_wlo, n_groups, r_pad, tmem_cols, n_seg, passes, d_vol, vol_div, row0, m, r,
-                col0, d_u);
+            for (int g0 = 0; g0 < n_groups; g0 += launch_groups) {
+                const int lg = (n_groups - g0) < launch_groups ? (n_groups - g0) : launch_groups;
+                project_tc_kernel<<<(unsigned)(rows_pad / kPjBM), kPjThreads, smem, st>>>(
+                    map_hi, map_lo, map_whi, map_wlo, g0, lg, r_pad, tmem_cols, n_seg < lg ? n_seg : lg, passes, d_vol,
+                    vol_div, row0, m, r, col0, g0 > 0, d_u);
+                note_launch(1);
+            }
             S3_LAUNCH_CHECK();
-            note_launch(2);
+            note_launch(1);
         }
         note_launch(1);
     }
