@@ -187,6 +187,25 @@ int s3_interp_gather(const void* d_data, int data_dtype, int64_t n_src, int64_t 
                      const int32_t* d_idx, const void* d_w, int64_t n_cells, int k,
                      const int32_t* d_out_row, void* d_out, int out_dtype, void* stream);
 
+/* ---- reconstruction error of a sampled grid --------------------------------------------------------
+ * the exported field `sampled` [n_sampled, n_comp, n_cols] is interpolated back onto the original points with the
+ * tables of the other direction (idx int32 / w fp32 [n_points, k]: the original points queried among the cell
+ * centres, in processing order; d_out_row int32 [n_points]: the original row of each, NULL = identity) and compared
+ * with `original` [n_points, n_comp, n_cols]:
+ *   r = sum_j w[p, j] * sampled[idx[p, j], d, t]   (fp32 FMA chain in neighbour order: the bits of the fp32 gather)
+ *   e = (double) r - (double) original[out_row[p], d, t]
+ * results, fp64 [n_comp, n_cols] each: d_sq_err = sum_p e^2, d_sq_ref = sum_p original^2, d_max_abs = max_p |e|;
+ * d_point_sq_err fp64 [n_points, n_comp] (optional, NULL = skipped): sum_t e^2 is ADDED into row out_row[p], so that
+ * successive time windows accumulate. Strides in elements and alignment rules as in s3_interp_gather_strided, both
+ * fields fp32 (anything else: S3_ERR_UNSUPPORTED). Every sum is reduced in a fixed order that depends on n_points only:
+ * the results are bit-identical from run to run, and each column's results do not depend on the other columns of the
+ * call (a time window gives the matching columns of the whole batch). 1 <= k <= 64.                      */
+int s3_recon_error(const void* d_sampled, int sampled_dtype, int64_t n_sampled, int n_comp, int64_t n_cols,
+                   int64_t s_row_stride, int64_t s_comp_stride, const void* d_original, int original_dtype,
+                   int64_t n_points, int64_t o_row_stride, int64_t o_comp_stride, const int32_t* d_idx,
+                   const float* d_w, const int32_t* d_out_row, int k, double* d_sq_err, double* d_sq_ref,
+                   double* d_max_abs, double* d_point_sq_err, void* stream);
+
 /* ---- streaming ingest -----------------------------------------------------------------------------
  * the reference feeds snapshot batches from host memory (export.py:128-167, utils.py:155-226). A window of the
  * time axis of a host field [rows, T] is a pitched 2-D region: one asynchronous copy per window and direction

@@ -67,6 +67,9 @@ _SIGNATURES = {
                                  c_void_p, c_int, c_void_p]),
     "s3_interp_gather_strided": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_int64, c_int64, c_void_p, c_void_p,
                                          c_int64, c_int, c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p]),
+    "s3_recon_error": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64,
+                               c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
+                               c_void_p, c_void_p]),
     "s3_copy2d_async": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64, c_int, c_void_p]),
     "s3_gather_rows": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int, c_void_p]),
     "s3_svd_row_means": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p]),

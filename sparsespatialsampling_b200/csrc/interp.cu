@@ -522,6 +522,224 @@ static int launch_interp(const void* data, const int32_t* idx, const void* w, in
     return S3_OK;
 }
 
+// ---- reconstruction error of a sampled grid (s3_recon_error) ----------------------------------------------------
+// The sampled field is gathered back onto the original points with the tables of the other direction (N original points
+// queried among the Nc cell centres) and compared there without materialising the [N, D, T] reconstruction:
+//   r = sum_j w[p, j] * sampled[idx[p, j], d, t]   (fp32 FMA chain in neighbour order: the gather's MODE 0 products)
+//   e = (double) r - (double) original[out_row[p], d, t]
+// Grid: one CTA per (point block, component, column tile), the tiles and components of one block adjacent in launch
+// order, so that they run together and the block's table rows and original rows are served from L2 to all of them. The
+// warps of a CTA walk the points of the block (warp w: points w, w + 8, ...; neighbouring points of the Morton order
+// share sampled rows, which L1 serves), each lane owns 8 columns of the 256-column tile. The fp64 column partials of the
+// warps are combined in shared memory in warp order, one partial per (block, column) goes to scratch and a second kernel
+// reduces them in block order. The reduction tree therefore depends on N only: the results are the same bits for any
+// CTA count (key 18) and for any set of other columns in the launch (a time window gives the full launch's columns).
+constexpr int kReconWarps = 8;          // warps per CTA
+constexpr int kReconBlock = 512;        // points per block: fixed, the order of every sum depends on it
+constexpr int kReconTile = 256;         // columns per tile: 32 lanes x 8
+constexpr int kReconGroup = 256;        // block partials per group of the first column-reduction pass
+static int g_recon_cap = 0;             // key 18: at most this many CTAs per (component, tile), 0 = no cap (tests)
+
+struct ReconGeom {
+    int64_t s_row, s_comp;              // sampled: elements between cells / between components
+    int64_t o_row, o_comp;              // original: elements between points / between components
+    int64_t n_cols;
+    int n_comp, n_tiles;
+};
+
+// WIDE: one 256-bit load per lane and row (base pointers and strides multiples of 32 bytes; a vector that straddles the
+// end of a row stays inside the 32-byte sector of the row's last column and its columns past the end are not used).
+// Otherwise the lane owns columns lane + 32 e with scalar loads, and nothing past a row is read.
+template <bool WIDE>
+__global__ void __launch_bounds__(kReconWarps * 32, 2)
+recon_error_kernel(const float* __restrict__ sampled, const float* __restrict__ original, const int32_t* __restrict__ idx,
+                   const float* __restrict__ w, const int32_t* __restrict__ out_row, int64_t n_points, int k,
+                   const ReconGeom g, int64_t n_blocks, int64_t n_slots, double* __restrict__ col_part,
+                   double* __restrict__ pt_part) {
+    __shared__ double s_red[3][kReconWarps][kReconTile];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int n_xt = g.n_comp * g.n_tiles;
+    const int xt = (int)(blockIdx.x % n_xt);
+    const int64_t slot = blockIdx.x / n_xt;
+    const int comp = xt / g.n_tiles, tile = xt % g.n_tiles;
+    const int64_t n_cols = g.n_cols, dt = (int64_t)g.n_comp * n_cols;
+    const int64_t tile0 = (int64_t)tile * kReconTile;
+    const float* s_base = sampled + (int64_t)comp * g.s_comp;
+    const float* o_base = original + (int64_t)comp * g.o_comp;
+    auto col_in_tile = [&](int e) { return WIDE ? lane * 8 + e : lane + 32 * e; };
+
+    for (int64_t pb = slot; pb < n_blocks; pb += n_slots) {
+        double se[8], sr[8], mx[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) se[e] = sr[e] = mx[e] = 0.0;
+        const int64_t p_end = min(n_points, (pb + 1) * kReconBlock);
+        for (int64_t p = pb * kReconBlock + warp; p < p_end; p += kReconWarps) {
+            int32_t idx_lo = 0, idx_hi = 0;
+            float w_lo = 0.f, w_hi = 0.f;
+            if (lane < k) { idx_lo = idx[p * k + lane]; w_lo = w[p * k + lane]; }
+            if (lane + 32 < k) { idx_hi = idx[p * k + lane + 32]; w_hi = w[p * k + lane + 32]; }
+            const int64_t orow = out_row ? (int64_t)out_row[p] : p;
+            const float* orig = o_base + orow * g.o_row;
+            float o[8], acc[8];
+#pragma unroll
+            for (int e = 0; e < 8; ++e) { o[e] = 0.f; acc[e] = 0.f; }
+            const int64_t c0 = tile0 + lane * 8;
+            if (WIDE) {
+                if (c0 < n_cols) {
+                    const Vec<float, 8> x = ld_vec<float, 8>(orig + c0);
+#pragma unroll
+                    for (int e = 0; e < 8; ++e) o[e] = x.v[e];
+                }
+            } else {
+#pragma unroll
+                for (int e = 0; e < 8; ++e) {
+                    const int64_t c = tile0 + col_in_tile(e);
+                    if (c < n_cols) o[e] = orig[c];
+                }
+            }
+#pragma unroll 4
+            for (int j = 0; j < k; ++j) {
+                const int32_t r = __shfl_sync(0xffffffffu, (j & 32) ? idx_hi : idx_lo, j & 31);
+                const float wj = __shfl_sync(0xffffffffu, (j & 32) ? w_hi : w_lo, j & 31);
+                const float* src = s_base + (int64_t)r * g.s_row;
+                if (WIDE) {
+                    if (c0 < n_cols) {
+                        const Vec<float, 8> x = ld_vec<float, 8>(src + c0);
+#pragma unroll
+                        for (int e = 0; e < 8; ++e) acc[e] = fmaf(wj, x.v[e], acc[e]);
+                    }
+                } else {
+#pragma unroll
+                    for (int e = 0; e < 8; ++e) {
+                        const int64_t c = tile0 + col_in_tile(e);
+                        if (c < n_cols) acc[e] = fmaf(wj, src[c], acc[e]);
+                    }
+                }
+            }
+            double ps = 0.0;                                  // sum over this lane's columns of e^2
+#pragma unroll
+            for (int e = 0; e < 8; ++e) {
+                if (tile0 + col_in_tile(e) < n_cols) {       // the n_cols % 8 tail of the last vector is not a column
+                    const double d = (double)acc[e] - (double)o[e];
+                    const double d2 = d * d;
+                    se[e] += d2;
+                    sr[e] += (double)o[e] * (double)o[e];
+                    mx[e] = fmax(mx[e], fabs(d));
+                    ps += d2;
+                }
+            }
+            if (pt_part) {
+#pragma unroll
+                for (int off = 16; off > 0; off >>= 1) ps += __shfl_xor_sync(0xffffffffu, ps, off);
+                if (lane == 0) pt_part[((int64_t)tile * n_points + p) * g.n_comp + comp] = ps;
+            }
+        }
+#pragma unroll
+        for (int e = 0; e < 8; ++e) {
+            s_red[0][warp][col_in_tile(e)] = se[e];
+            s_red[1][warp][col_in_tile(e)] = sr[e];
+            s_red[2][warp][col_in_tile(e)] = mx[e];
+        }
+        __syncthreads();
+        const int t = threadIdx.x;
+        if (tile0 + t < n_cols) {
+            double a = 0.0, b = 0.0, m = 0.0;
+#pragma unroll
+            for (int q = 0; q < kReconWarps; ++q) {
+                a += s_red[0][q][t];
+                b += s_red[1][q][t];
+                m = fmax(m, s_red[2][q][t]);
+            }
+            double* part = col_part + pb * 3 * dt + (int64_t)comp * n_cols + tile0 + t;
+            part[0] = a;
+            part[dt] = b;
+            part[2 * dt] = m;
+        }
+        __syncthreads();
+    }
+}
+
+// in: rows of [3][dt] partials (sum, sum, max); group y reduces rows [y * rows_per_group, ...) in row order into
+// out{0,1,2}[y * ld_out + c]
+__global__ void recon_reduce_cols_kernel(const double* __restrict__ in, int64_t n_rows, int64_t rows_per_group,
+                                         int64_t dt, double* out0, double* out1, double* out2, int64_t ld_out) {
+    const int64_t c3 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c3 >= 3 * dt) return;
+    const int plane = (int)(c3 / dt);
+    const int64_t c = c3 % dt;
+    const int64_t r0 = (int64_t)blockIdx.y * rows_per_group;
+    const int64_t r1 = min(n_rows, r0 + rows_per_group);
+    double acc = 0.0;
+    for (int64_t r = r0; r < r1; ++r) {
+        const double v = in[r * 3 * dt + c3];
+        acc = plane == 2 ? fmax(acc, v) : acc + v;
+    }
+    double* out = plane == 0 ? out0 : plane == 1 ? out1 : out2;
+    out[blockIdx.y * ld_out + c] = acc;
+}
+
+// point_sq_err[out_row[p], d] += sum over the tiles, in tile order, of the (point, tile) partials
+__global__ void recon_reduce_points_kernel(const double* __restrict__ pt_part, int64_t n_points, int n_comp, int n_tiles,
+                                           const int32_t* __restrict__ out_row, double* __restrict__ point_sq_err) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t n = n_points * n_comp;
+    if (i >= n) return;
+    double s = 0.0;
+    for (int t = 0; t < n_tiles; ++t) s += pt_part[(int64_t)t * n + i];
+    const int64_t p = i / n_comp;
+    const int64_t orow = out_row ? (int64_t)out_row[p] : p;
+    point_sq_err[orow * n_comp + i % n_comp] += s;
+}
+
+static int launch_recon_error(const float* sampled, const float* original, const int32_t* idx, const float* w,
+                              const int32_t* out_row, int64_t n_points, int k, ReconGeom g, double* sq_err,
+                              double* sq_ref, double* max_abs, double* point_sq_err, cudaStream_t stream) {
+    const int64_t dt = (int64_t)g.n_comp * g.n_cols;
+    const int64_t n_blocks = ceil_div(n_points, kReconBlock);
+    const int64_t n_xt = (int64_t)g.n_comp * g.n_tiles;
+    int64_t n_slots = n_blocks;
+    if (g_recon_cap > 0 && n_slots > g_recon_cap) n_slots = g_recon_cap;
+    S3_REQUIRE(n_xt * n_slots < ((int64_t)1 << 31), "s3_recon_error: too many CTAs (%lld tiles x %lld blocks)",
+               (long long)n_xt, (long long)n_slots);
+    const int64_t n_groups = ceil_div(n_blocks, kReconGroup);
+    S3_REQUIRE(n_groups <= 65535, "s3_recon_error: too many points (%lld)", (long long)n_points);
+    Scratch scratch(stream);
+    double *col_part = nullptr, *grp_part = nullptr, *pt_part = nullptr;
+    S3_TRY(scratch.alloc(&col_part, (size_t)(n_blocks * 3 * dt)));
+    if (point_sq_err) S3_TRY(scratch.alloc(&pt_part, (size_t)(g.n_tiles * n_points * g.n_comp)));
+    const bool wide = (uintptr_t)sampled % 32 == 0 && (uintptr_t)original % 32 == 0 && g.s_row % 8 == 0 &&
+                      g.s_comp % 8 == 0 && g.o_row % 8 == 0 && g.o_comp % 8 == 0;
+    const unsigned ctas = (unsigned)(n_xt * n_slots);
+    if (wide)
+        recon_error_kernel<true><<<ctas, kReconWarps * 32, 0, stream>>>(sampled, original, idx, w, out_row, n_points, k,
+                                                                         g, n_blocks, n_slots, col_part, pt_part);
+    else
+        recon_error_kernel<false><<<ctas, kReconWarps * 32, 0, stream>>>(sampled, original, idx, w, out_row, n_points, k,
+                                                                          g, n_blocks, n_slots, col_part, pt_part);
+    S3_LAUNCH_CHECK();
+    const unsigned col_ctas = (unsigned)ceil_div(3 * dt, 256);
+    if (n_groups == 1) {
+        recon_reduce_cols_kernel<<<dim3(col_ctas, 1), 256, 0, stream>>>(col_part, n_blocks, n_blocks, dt, sq_err,
+                                                                         sq_ref, max_abs, 0);
+        S3_LAUNCH_CHECK();
+    } else {
+        S3_TRY(scratch.alloc(&grp_part, (size_t)(n_groups * 3 * dt)));
+        recon_reduce_cols_kernel<<<dim3(col_ctas, (unsigned)n_groups), 256, 0, stream>>>(
+            col_part, n_blocks, kReconGroup, dt, grp_part, grp_part + dt, grp_part + 2 * dt, 3 * dt);
+        S3_LAUNCH_CHECK();
+        recon_reduce_cols_kernel<<<dim3(col_ctas, 1), 256, 0, stream>>>(grp_part, n_groups, n_groups, dt, sq_err,
+                                                                         sq_ref, max_abs, 0);
+        S3_LAUNCH_CHECK();
+    }
+    if (point_sq_err) {
+        recon_reduce_points_kernel<<<(unsigned)ceil_div(n_points * g.n_comp, 256), 256, 0, stream>>>(
+            pt_part, n_points, g.n_comp, g.n_tiles, out_row, point_sq_err);
+        S3_LAUNCH_CHECK();
+    }
+    note_launch(point_sq_err ? (n_groups == 1 ? 3 : 4) : (n_groups == 1 ? 2 : 3));
+    return S3_OK;
+}
+
 }  // namespace s3
 
 using namespace s3;
@@ -548,6 +766,7 @@ extern "C" int s3x_tune(int key, int value) {
         case 11: S3_REQUIRE(value >= 1 && value <= (1 << 20), "s3x_tune: segments per fp64 flush must be >= 1"); g_tc_flush_segments = value; return S3_OK;
         case 14: S3_REQUIRE(value == 0 || value == 1, "s3x_tune: paired Gram kernel must be 0 or 1"); g_tc_pair = value; return S3_OK;
         case 17: S3_REQUIRE(value >= 0, "s3x_tune: plane-row cap must be 0 (none) or >= 1"); g_plane_rows_cap = value; return S3_OK;
+        case 18: S3_REQUIRE(value >= 0, "s3x_tune: reconstruction-error CTA cap must be 0 (none) or >= 1"); g_recon_cap = value; return S3_OK;
     }
     s3::set_error("s3x_tune: unknown key %d", key);
     return S3_ERR_INVALID;
@@ -589,6 +808,45 @@ extern "C" int s3_interp_gather_strided(const void* d_data, int data_dtype, int6
         return launch_interp<double, double, double, 1>(d_data, d_idx, d_w, n_cells, k, d_out_row, d_out, n_comp, g, st);
     s3::set_error("s3_interp_gather: unsupported dtype combination data=%d out=%d", data_dtype, out_dtype);
     return S3_ERR_UNSUPPORTED;
+}
+
+extern "C" int s3_recon_error(const void* d_sampled, int sampled_dtype, int64_t n_sampled, int n_comp, int64_t n_cols,
+                              int64_t s_row_stride, int64_t s_comp_stride, const void* d_original, int original_dtype,
+                              int64_t n_points, int64_t o_row_stride, int64_t o_comp_stride, const int32_t* d_idx,
+                              const float* d_w, const int32_t* d_out_row, int k, double* d_sq_err, double* d_sq_ref,
+                              double* d_max_abs, double* d_point_sq_err, void* stream) {
+    S3_REQUIRE(n_points >= 0 && n_cols >= 0 && n_comp >= 0 && n_sampled >= 0, "s3_recon_error: bad sizes");
+    if (sampled_dtype != S3_F32 || original_dtype != S3_F32) {
+        s3::set_error("s3_recon_error: fields must be fp32 (sampled dtype %d, original dtype %d); the error of fp64 "
+                      "fields is not implemented", sampled_dtype, original_dtype);
+        return S3_ERR_UNSUPPORTED;
+    }
+    S3_REQUIRE(k >= 1 && k <= 64, "s3_recon_error: k=%d out of range [1, 64]", k);
+    if (n_cols == 0 || n_comp == 0) return S3_OK;
+    S3_REQUIRE(d_sq_err && d_sq_ref && d_max_abs, "s3_recon_error: NULL result");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (n_points == 0) {                    // no points: zero sums, nothing added to the point map
+        const size_t bytes = (size_t)n_comp * n_cols * sizeof(double);
+        S3_CUDA(cudaMemsetAsync(d_sq_err, 0, bytes, st));
+        S3_CUDA(cudaMemsetAsync(d_sq_ref, 0, bytes, st));
+        S3_CUDA(cudaMemsetAsync(d_max_abs, 0, bytes, st));
+        return S3_OK;
+    }
+    S3_REQUIRE(d_sampled && d_original && d_idx && d_w, "s3_recon_error: NULL argument");
+    S3_REQUIRE(n_sampled >= 1, "s3_recon_error: no sampled cells");
+    S3_REQUIRE((s_comp_stride >= n_cols && o_comp_stride >= n_cols) || n_comp == 1,
+               "s3_recon_error: component stride smaller than a row");
+    S3_REQUIRE(s_row_stride >= (n_comp - 1) * s_comp_stride + n_cols && o_row_stride >= (n_comp - 1) * o_comp_stride + n_cols,
+               "s3_recon_error: row stride smaller than a row");
+    ReconGeom g{};
+    g.s_row = s_row_stride; g.s_comp = n_comp == 1 ? 0 : s_comp_stride;
+    g.o_row = o_row_stride; g.o_comp = n_comp == 1 ? 0 : o_comp_stride;
+    g.n_cols = n_cols;
+    g.n_comp = n_comp;
+    g.n_tiles = (int)ceil_div(n_cols, kReconTile);
+    S3_REQUIRE(ceil_div(n_cols, kReconTile) * n_comp < (1 << 20), "s3_recon_error: too many columns");
+    return launch_recon_error(reinterpret_cast<const float*>(d_sampled), reinterpret_cast<const float*>(d_original),
+                              d_idx, d_w, d_out_row, n_points, k, g, d_sq_err, d_sq_ref, d_max_abs, d_point_sq_err, st);
 }
 
 extern "C" int s3_interp_gather(const void* d_data, int data_dtype, int64_t n_src, int64_t row_len,
