@@ -6,17 +6,15 @@ import numpy as np
 
 def write_binary_stl(path, triangles):
     tri = np.asarray(triangles, dtype=np.float32)
+    n = np.cross(tri[:, 1] - tri[:, 0], tri[:, 2] - tri[:, 0])
+    nn = np.linalg.norm(n, axis=1, keepdims=True)
+    rec = np.zeros(tri.shape[0], dtype=np.dtype([("n", "<f4", 3), ("v", "<f4", (3, 3)), ("a", "<u2")]))
+    rec["n"] = np.where(nn > 0, n / np.where(nn > 0, nn, 1), n)
+    rec["v"] = tri
     with open(path, "wb") as f:
         f.write(b"s3b200 test mesh".ljust(80, b" "))
         f.write(struct.pack("<I", tri.shape[0]))
-        for t in tri:
-            n = np.cross(t[1] - t[0], t[2] - t[0])
-            nn = np.linalg.norm(n)
-            n = n / nn if nn > 0 else n
-            f.write(struct.pack("<3f", *n))
-            for v in t:
-                f.write(struct.pack("<3f", *v))
-            f.write(struct.pack("<H", 0))
+        f.write(rec.tobytes())
 
 
 def cube_triangles(lo=(0.0, 0.0, 0.0), hi=(1.0, 1.0, 1.0)):
