@@ -63,16 +63,14 @@ int s3_morton_order(const double* d_coords, int64_t n, int dim, int32_t* d_perm,
 
 /* ---- refinement engine (device side of SamplingTree, sparseSpatialSampling/s_cube.py) -------------
  * Cell state: structure of arrays indexed by the reference's cell index (creation order):
- *   d_center fp64 [cap, dim], d_level int32 [cap], d_lattice int32 [cap, dim] (integer position of the
- *   cell at its own level), d_gain fp64 [cap], d_metric fp64 [cap], d_flags uint8 [cap]
- *   (bit 0 = leaf, bit 1 = invalid / removed by a geometry).                                         */
+ *   d_center fp64 [cap, dim], d_level int32 [cap], d_gain fp64 [cap], d_metric fp64 [cap],
+ *   d_flags uint8 [cap] (bit 0 = leaf, bit 1 = invalid / removed by a geometry).                     */
 
 /* children of `d_parents[i]` get indices first_child + i*2^dim + c, c in CH order
  * (s_cube.py:29,188-194); centre = fl(parent + dir * 0.25*width/2^level) (s_cube.py:399-445,865-902);
  * parents lose, children get the leaf flag (_update_leaf_cells, s_cube.py:243-251)                 */
-int s3_cells_refine(double* d_center, int32_t* d_level, int32_t* d_lattice, uint8_t* d_flags,
-                    const int64_t* d_parents, int64_t n_parents, int64_t first_child, int dim,
-                    double width, void* stream);
+int s3_cells_refine(double* d_center, int32_t* d_level, uint8_t* d_flags, const int64_t* d_parents,
+                    int64_t n_parents, int64_t first_child, int dim, double width, void* stream);
 
 /* SamplingTree._update_gain (s_cube.py:207-241) + numba _update_gain (s_cube.py:1840-1859):
  * KNN/IDW metric at the cell centre and at the 2^dim would-be child centres, sum|m0-mj|, gain.
@@ -116,14 +114,6 @@ int s3_select_topk(const double* d_gain, const uint8_t* d_flags, int64_t n_cells
                    int64_t* d_out, void* stream);
 /* implementation switch (tests / benchmarking): 1 = one cooperative launch for k <= 8192 (default), 0 = multi-kernel */
 int s3_select_set_fused(int on);
-
-/* final grid assembly (_resort_nodes_and_indices_of_grid, s_cube.py:734-772): corners of the leaf cells
- * `d_leaves` (int64 [n_leaves], output order) de-duplicated on the finest lattice.
- * d_faces int32 [n_leaves, 2^dim] (corner order CH), d_vertices fp64 [>= n_leaves*2^dim, dim] (first
- * *n_vertices rows are valid). Synchronises `stream`.                                               */
-int s3_build_nodes(const int64_t* d_leaves, int64_t n_leaves, const double* d_center,
-                   const int32_t* d_level, const int32_t* d_lattice, int dim, int max_level, double width,
-                   int32_t* d_faces, double* d_vertices, int64_t* n_vertices, void* stream);
 
 /* ---- cell topology (HOST side, plain integer bookkeeping; all pointers are host pointers) -----------
  * The reference's neighbour pointers and shared node ids are history dependent (see csrc/topology.cu); this

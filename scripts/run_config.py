@@ -78,7 +78,6 @@ def main(tmp_dir: str):
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--tune", default="", help="comma separated key=value pairs for s3x_tune (csrc/interp.cu), e.g. 2=1,3=0")
     ap.add_argument("--dense", action="store_true", help="the reference's dense [N, D, T] layout instead of 128-byte pitched rows")
-    ap.add_argument("--lattice-vertices", action="store_true", help="exact_topology=False")
     ap.add_argument("--stl-subdiv", type=int, default=4, help="C5: icosphere subdivisions of the STL body (4: 5120 triangles, 6: 81920)")
     ap.add_argument("--grid-only", action="store_true", help="stop after grid generation (timings only)")
     ap.add_argument("--e2e", action="store_true", help="also time the host-to-host export (256 snapshots): DMA vs row gather")
@@ -99,8 +98,7 @@ def main(tmp_dir: str):
 
     # ---- grid generation
     t0 = time.time()
-    sc = s3.SparseSpatialSampling(x, metric, geoms, tmp_dir, args.name.lower(), **grid_kw,
-                                  exact_topology=not args.lattice_vertices)
+    sc = s3.SparseSpatialSampling(x, metric, geoms, tmp_dir, args.name.lower(), **grid_kw)
     t_setup = time.time() - t0
     sc.execute_grid_generation()
     info = sc.mesh_info

@@ -36,8 +36,7 @@ _SIGNATURES = {
     "s3_knn_predict": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "s3_knn_tables": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "s3_morton_order": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
-    "s3_cells_refine": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_double,
-                                c_void_p]),
+    "s3_cells_refine": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_double, c_void_p]),
     "s3_cells_gain": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_double, c_double, c_int,
                               c_void_p, c_void_p, c_void_p]),
     "s3_cells_mask": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_double, c_void_p, c_void_p, c_int,
@@ -48,8 +47,6 @@ _SIGNATURES = {
                                  c_void_p]),
     "s3_select_topk": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "s3_select_set_fused": (c_int, [c_int]),
-    "s3_build_nodes": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int, c_int, c_double, c_void_p, c_void_p,
-                               POINTER(c_int64), c_void_p]),
     "s3_topo_create": (c_int, [c_int, c_void_p, c_double, c_int, POINTER(c_void_p)]),
     "s3_topo_sync": (c_int, [c_void_p]),
     "s3_topo_free": (c_int, [c_void_p]),

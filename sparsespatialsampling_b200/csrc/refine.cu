@@ -1,8 +1,7 @@
 // Level-synchronous octree/quadtree refinement kernels (device side of SamplingTree, s_cube.py).
 //
 // Cell state is a structure of arrays indexed by the reference's cell index (creation order):
-//   center fp64 [cap, dim], level int32 [cap], lattice int32 [cap, dim] (integer position at the
-//   cell's own level), gain fp64 [cap], metric fp64 [cap], flags uint8 [cap].
+//   center fp64 [cap, dim], level int32 [cap], gain fp64 [cap], metric fp64 [cap], flags uint8 [cap].
 #include "common.cuh"
 #include "geometry.cuh"
 #include "stl.cuh"
@@ -28,9 +27,8 @@ __device__ __forceinline__ void direction(int dim, int c, int* d) {
 
 // ---------------------------------------------------------------- children (s_cube.py:399-445, :865-902)
 __global__ void __launch_bounds__(256)
-cells_refine_kernel(double* __restrict__ center, int32_t* __restrict__ level, int32_t* __restrict__ lattice,
-                    uint8_t* __restrict__ flags, const int64_t* __restrict__ parents, int64_t n_parents,
-                    int64_t first_child, int dim, double width) {
+cells_refine_kernel(double* __restrict__ center, int32_t* __restrict__ level, uint8_t* __restrict__ flags,
+                    const int64_t* __restrict__ parents, int64_t n_parents, int64_t first_child, int dim, double width) {
     const int nch = 1 << dim;
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n_parents * nch) return;
@@ -46,7 +44,6 @@ cells_refine_kernel(double* __restrict__ center, int32_t* __restrict__ level, in
     for (int a = 0; a < dim; ++a) {
         const double pc = center[p * dim + a];
         center[child * dim + a] = __dadd_rn(pc, d[a] > 0 ? off : -off);
-        lattice[child * dim + a] = 2 * lattice[p * dim + a] + (d[a] > 0 ? 1 : 0);
     }
     level[child] = lp + 1;
     flags[child] = kFlagLeaf;
@@ -627,15 +624,14 @@ using namespace s3;
 
 extern "C" {
 
-int s3_cells_refine(double* d_center, int32_t* d_level, int32_t* d_lattice, uint8_t* d_flags,
-                    const int64_t* d_parents, int64_t n_parents, int64_t first_child, int dim, double width,
-                    void* stream) {
-    S3_REQUIRE(d_center && d_level && d_lattice && d_flags && d_parents, "s3_cells_refine: NULL argument");
+int s3_cells_refine(double* d_center, int32_t* d_level, uint8_t* d_flags, const int64_t* d_parents, int64_t n_parents,
+                    int64_t first_child, int dim, double width, void* stream) {
+    S3_REQUIRE(d_center && d_level && d_flags && d_parents, "s3_cells_refine: NULL argument");
     S3_REQUIRE(dim == 2 || dim == 3, "s3_cells_refine: dim must be 2 or 3");
     if (n_parents == 0) return S3_OK;
     const int64_t threads = n_parents << dim;
     cells_refine_kernel<<<(unsigned)ceil_div(threads, 256), 256, 0, (cudaStream_t)stream>>>(
-        d_center, d_level, d_lattice, d_flags, d_parents, n_parents, first_child, dim, width);
+        d_center, d_level, d_flags, d_parents, n_parents, first_child, dim, width);
     S3_LAUNCH_CHECK();
     note_launch(1);
     return S3_OK;

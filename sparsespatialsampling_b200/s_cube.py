@@ -17,7 +17,6 @@ host (this file)       the sequential control flow of the reference (stopping cr
 Per iteration the host reads back: the k selected cell indices, one invalid flag per new cell, one scalar
 (sum of squared leaf metrics).
 """
-import ctypes
 import logging
 from time import time
 from typing import Union
@@ -70,13 +69,8 @@ class SamplingTree(object):
                  uniform_level: int = 5, min_metric: float = 0.75, max_delta_level: bool = False,
                  n_cells_iter_start: int = None, n_cells_iter_end: int = None, n_jobs: int = 1,
                  relTol: Union[int, float] = 1e-3, reach_at_least: float = 0.75, pre_select: bool = False,
-                 device=None, sdm_order: int = None, exact_topology: bool = True):
+                 device=None, sdm_order: int = None):
         _lib.require_cuda()
-        # exact_topology: replay the reference's neighbour pointers / node ids on the host (topology.py) -- the
-        # reference's vertex numbering and max_delta_level closure are history dependent. False: vertices from a
-        # lattice de-duplication on the device and a geometric max_delta_level closure (same cells / centres / levels,
-        # different vertex numbering).
-        self._exact_topology = bool(exact_topology)
         self._topo = None
         self._lib = _lib.load()
         self._device = pt.device(device) if device is not None else pt.device("cuda", pt.cuda.current_device())
@@ -104,18 +98,6 @@ class SamplingTree(object):
         self._nch = 2 ** self._n_dimensions
         self._sdm_order = probe_sum_order_8() if sdm_order is None else int(sdm_order)
 
-        # neighbour directions in the reference's NB order (s_cube.py:22-26): same plane w, nw, n, ne, e, se, s, sw;
-        # 3-D adds the lower plane (z-1: same eight + centre) and then the upper plane (z+1)
-        plane = [(-1, 0), (-1, 1), (0, 1), (1, 1), (1, 0), (1, -1), (0, -1), (-1, -1)]
-        if self._n_dimensions == 2:
-            self._nb_dirs = [np.array(p, dtype=np.int64) for p in plane]
-        else:
-            self._nb_dirs = ([np.array(p + (0,), dtype=np.int64) for p in plane] +
-                             [np.array(p + (-1,), dtype=np.int64) for p in plane + [(0, 0)]] +
-                             [np.array(p + (1,), dtype=np.int64) for p in plane + [(0, 0)]])
-        # (level, lattice coords) -> cell index, only for the geometric closure
-        self._cell_lookup = {} if (max_delta_level and not exact_topology) else None
-
         # KNN index over the original grid with the metric as regression target (s_cube.py:161-163)
         t0 = time()
         with pt.cuda.device(self._device):
@@ -141,10 +123,9 @@ class SamplingTree(object):
 
         # device state
         self._cap = 0
-        self._center = self._level = self._lattice = self._gain = self._metric_d = self._flags = None
+        self._center = self._level = self._gain = self._metric_d = self._flags = None
         self._levels_h = np.zeros(0, dtype=np.int32)
         self._invalid_h = np.zeros(0, dtype=bool)
-        self._lattice_h = np.zeros((0, self._n_dimensions), dtype=np.int64)
         self._scalar = pt.zeros(1, dtype=pt.float64, device=self._device)
         # pinned staging of the per-iteration transfers: parent list up, (invalid flags, captured-metric sum) down with
         # ONE synchronisation per iteration
@@ -168,11 +149,6 @@ class SamplingTree(object):
         self._target_norm = float(np.sqrt(self._sumsq(tgt)))
 
     # ------------------------------------------------------------------------------------------ helpers
-    def _topo_call(self, fn, *args) -> None:
-        """Topology update: applied at once with max_delta_level (the closure reads the pointers), otherwise queued on
-        the library's native worker thread and applied next to the device work (Topology(asynchronous=True))."""
-        fn(*args)
-
     def _stream(self):
         # the C-ABI calls of one refine() run are all queued on the stream that was current when it started
         # (torch.cuda.current_stream() costs ~15 us per call -- more than a small launch)
@@ -213,7 +189,6 @@ class SamplingTree(object):
         self._ptr_cache = {}
         self._center = grow(self._center, (new_cap, d), pt.float64)
         self._level = grow(self._level, (new_cap,), pt.int32)
-        self._lattice = grow(self._lattice, (new_cap, d), pt.int32)
         self._gain = grow(self._gain, (new_cap,), pt.float64)
         self._metric_d = grow(self._metric_d, (new_cap,), pt.float64)
         self._flags = grow(self._flags, (new_cap,), pt.uint8)
@@ -223,9 +198,6 @@ class SamplingTree(object):
         iv = np.zeros(new_cap, dtype=bool)
         iv[:self._invalid_h.size] = self._invalid_h
         self._invalid_h = iv
-        la = np.zeros((new_cap, d), dtype=np.int64)
-        la[:self._lattice_h.shape[0]] = self._lattice_h
-        self._lattice_h = la
         self._cap = new_cap
 
     # ------------------------------------------------------------------------------------------ root cell
@@ -263,17 +235,13 @@ class SamplingTree(object):
         self._reserve(1)
         self._center[0] = centers_[0].to(self._device)
         self._level[0] = 0
-        self._lattice[0] = 0
         self._gain[0] = self._gain0
         self._metric_d[0] = float(metric[0])
         self._flags[0] = FLAG_LEAF
         self._n_cells = 1
         self._leaf_cells.add(0)
-        if self._cell_lookup is not None:
-            self._cell_lookup[(0,) + (0,) * d] = 0
-        if self._exact_topology:
-            # without max_delta_level nothing reads the pointers before the final grid assembly
-            self._topo = Topology(d, centers_[0].numpy(), self._width, asynchronous=self.topology_async and not self._max_delta_level)
+        # without max_delta_level nothing reads the pointers before the final grid assembly
+        self._topo = Topology(d, centers_[0].numpy(), self._width, asynchronous=self.topology_async and not self._max_delta_level)
 
     # ------------------------------------------------------------------------------------------ refinement
     def _refine_cells(self, parents: list) -> range:
@@ -292,25 +260,14 @@ class SamplingTree(object):
         par_d = self._pin_i64[:n_par].to(self._device, non_blocking=True)
         if self._stream_obj is None:
             pt.cuda.set_device(self._device)
-        _lib.check(self._lib.s3_cells_refine(self._p("_center"), self._p("_level"), self._p("_lattice"),
-                                             self._p("_flags"), _lib.ptr(par_d), n_par, first, self._n_dimensions,
-                                             self._width, self._stream()))
+        _lib.check(self._lib.s3_cells_refine(self._p("_center"), self._p("_level"), self._p("_flags"), _lib.ptr(par_d),
+                                             n_par, first, self._n_dimensions, self._width, self._stream()))
         _lib.check(self._lib.s3_cells_gain(self._knn.handle, self._p("_center"), self._p("_level"), None, first, n_new,
                                            self._k, self._width, self._gain0, self._sdm_order, self._p("_metric_d"),
                                            self._p("_gain"), self._stream()))
         self._levels_h[first:first + n_new] = np.repeat(self._levels_h[par_h] + 1, self._nch)
-        if self._topo is not None and n_par:
-            self._topo_call(self._topo.refine, par_h.copy())   # host replay of _assign_neighbors + _assign_indices
-        if self._cell_lookup is not None and n_par:
-            # host mirror of the integer lattice position (child = 2 * parent + [direction > 0]) for neighbour look-ups
-            d = self._n_dimensions
-            pos = (self._child_dirs() > 0).astype(np.int64)                                    # [2^d, d]
-            lat = (2 * self._lattice_h[par_h][:, None, :] + pos[None, :, :]).reshape(-1, d)
-            self._lattice_h[first:first + n_new] = lat
-            lv = self._levels_h[first:first + n_new]
-            for t in range(n_new):
-                self._cell_lookup[(int(lv[t]),) + tuple(int(v) for v in lat[t])] = first + t
         if n_par:
+            self._topo.refine(par_h.copy())                   # host replay of _assign_neighbors + _assign_indices
             self._current_max_level = max(self._current_max_level, int(self._levels_h[par_h].max()) + 1)
 
         # leaf-set bookkeeping exactly as the reference does it (s_cube.py:877-899, :243-251): the reference fills
@@ -323,39 +280,14 @@ class SamplingTree(object):
         self._n_cells += n_new
         return range(first, first + n_new)
 
-    def _child_dirs(self) -> np.ndarray:
-        if self._n_dimensions == 2:
-            return np.array([[-1, -1], [-1, 1], [1, 1], [1, -1]], dtype=np.int64)
-        return np.array([[-1, -1, 1], [-1, 1, 1], [1, 1, 1], [1, -1, 1], [-1, -1, -1], [-1, 1, -1], [1, 1, -1],
-                         [1, -1, -1]], dtype=np.int64)
-
     # ------------------------------------------------------------------------------------------ delta-level constraint
     def _check_nb(self, _cell_no: int) -> list:
         """
         Leaf neighbours of a cell (8 / 26 directions, reference order) with a lower level: refining the cell alone would
-        create a level difference of two (s_cube.py:447-464). The neighbour in a direction is the leaf covering the
-        adjacent same-level lattice position -- the geometric meaning of the reference's neighbour pointers. With
-        ``exact_topology`` the reference's own (possibly stale) pointers are replayed instead.
+        create a level difference of two (s_cube.py:447-464), read from the host replay of the reference's own (possibly
+        stale) neighbour pointers.
         """
-        if self._topo is not None:
-            return self._topo.check_nb(_cell_no)
-        lv = int(self._levels_h[_cell_no])
-        pos = self._lattice_h[_cell_no]
-        out = []
-        for dvec in self._nb_dirs:
-            q = pos + dvec
-            if (q < 0).any() or (q >= (1 << lv)).any():
-                continue
-            for up in range(0, lv + 1):
-                key = (lv - up,) + tuple(int(v) >> up for v in q)
-                c = self._cell_lookup.get(key)
-                if c is None:
-                    continue
-                # first existing ancestor-or-self of the adjacent position: a coarser leaf forces refinement
-                if up > 0 and c in self._leaf_cells:
-                    out.append(c)
-                break
-        return out
+        return self._topo.check_nb(_cell_no)
 
     def _check_constraint(self, nb_violating_constraint: set) -> set:
         # s_cube.py:466-506: transitive closure of the constraint over the neighbours that get refined as well
@@ -363,8 +295,7 @@ class SamplingTree(object):
         while new_cells_to_check:
             tmp = set()
             for c in nb_violating_constraint:
-                if self._topo is not None:
-                    self._topo.refresh_siblings([c])          # s_cube.py:489-490
+                self._topo.refresh_siblings([c])              # s_cube.py:489-490
                 tmp.update(self._check_nb(c))
             if not tmp or tmp.issubset(nb_violating_constraint):
                 new_cells_to_check = False
@@ -482,8 +413,7 @@ class SamplingTree(object):
             return _idx
         for c in _idx:
             self._invalid_h[c] = True
-        if self._topo is not None:
-            self._topo_call(self._topo.mark_invalid, list(_idx))   # neighbour reset, s_cube.py:721-731
+        self._topo.mark_invalid(list(_idx))                  # neighbour reset, s_cube.py:721-731
         self._leaf_cells -= _idx
         return None
 
@@ -495,8 +425,7 @@ class SamplingTree(object):
             logger.info(f"\r\tStarting iteration no. {j}, N_cells = {len(self._leaf_cells)}")
             parents = list(self._leaf_cells)
             new_cells = self._refine_cells(parents)
-            if self._topo is not None:
-                self._topo_call(self._topo.refresh_children, parents)   # second pass, s_cube.py:547-549
+            self._topo.refresh_children(parents)             # second pass, s_cube.py:547-549
             self._current_min_level += 1
             self._remove_invalid_cells(new_cells)
         self._current_max_level = max(self._current_max_level, self._min_level)
@@ -580,14 +509,13 @@ class SamplingTree(object):
             if self._selected_log is not None:
                 self._selected_log.append(list(_leaf_cells_sorted))
             to_refine = set()
-            if self._topo is not None and not self._max_delta_level:
+            if not self._max_delta_level:
                 # s_cube.py:611 for every selected cell; nothing reads the pointers in between, so one call
-                self._topo_call(self._topo.refresh_siblings, list(_leaf_cells_sorted))
+                self._topo.refresh_siblings(list(_leaf_cells_sorted))
             for i in _leaf_cells_sorted:
                 to_refine.add(i)
                 if self._max_delta_level:
-                    if self._topo is not None:
-                        self._topo.refresh_siblings([i])      # s_cube.py:611
+                    self._topo.refresh_siblings([i])          # s_cube.py:611
                     nb_to_refine_as_well = set(self._check_nb(i))
                     to_refine.update(self._check_constraint(nb_to_refine_as_well))
             self._fuse_metric = self._n_cells_max is None
@@ -659,18 +587,17 @@ class SamplingTree(object):
                         continue
                     if self._levels_h[i] < _global_max_level:
                         to_refine.add(i)
-                        if self._topo is not None:            # s_cube.py:826
-                            if self._max_delta_level:
-                                self._topo.refresh_siblings([i])
-                            else:
-                                refresh.append(i)             # nothing reads the pointers inside this loop
+                        if self._max_delta_level:             # s_cube.py:826
+                            self._topo.refresh_siblings([i])
+                        else:
+                            refresh.append(i)                 # nothing reads the pointers inside this loop
                     if self._max_delta_level:
                         nb_to_refine_as_well = set(self._check_nb(i))
                         nb_to_refine_as_well.update(self._check_constraint(nb_to_refine_as_well))
                         to_refine.update(nb_to_refine_as_well)
                         checked.update(nb_to_refine_as_well)
                 if refresh:
-                    self._topo_call(self._topo.refresh_siblings, refresh)
+                    self._topo.refresh_siblings(refresh)
                 new_cells = self._refine_cells(list(to_refine))
                 _idx_new = {c for c in new_cells}
                 # children are only tested against the geometry being refined (s_cube.py:850)
@@ -697,35 +624,16 @@ class SamplingTree(object):
         if leaf_order != ascending:
             logger.warning("Leaf-set iteration order differs from ascending cell index; 'centers' and 'faces' follow "
                            "the reference's two different orders.")
-        n_leaf = len(leaf_order)
-        d = self._n_dimensions
         order_d = pt.tensor(leaf_order, dtype=pt.int64, device=self._device)
-        if self._topo is not None:
-            # the reference's node table: shared ids from the replayed pointers, unused ids squeezed out (:750-771)
-            self._topo.sync()
-            faces, vertices, _ = self._topo.final()
-            assert faces.shape[0] == n_leaf, "host topology and device cell state disagree on the leaf cells"
-            self.face_ids = pt.from_numpy(faces)
-            self.all_nodes = pt.from_numpy(vertices)
-            self.all_centers = self._center[order_d].cpu()
-            self.all_levels = self._level[order_d].to(pt.int64).cpu().unsqueeze(-1)
-            self._topo = None                                 # native handle: not part of the pickled object
-            self._times["t_end_renumber"] = time()
-            return
-        asc_d = order_d if leaf_order == ascending else pt.tensor(ascending, dtype=pt.int64, device=self._device)
-        max_level = int(self._levels_h[np.asarray(ascending, dtype=np.int64)].max())
-        faces = pt.empty((n_leaf, self._nch), dtype=pt.int32, device=self._device)
-        vertices = pt.empty((n_leaf * self._nch, d), dtype=pt.float64, device=self._device)
-        n_vert = ctypes.c_int64(0)
-        with pt.cuda.device(self._device):
-            _lib.check(self._lib.s3_build_nodes(_lib.ptr(asc_d), n_leaf, _lib.ptr(self._center), _lib.ptr(self._level),
-                                                _lib.ptr(self._lattice), d, max_level, self._width, _lib.ptr(faces),
-                                                _lib.ptr(vertices), ctypes.byref(n_vert), self._stream()))
-        self.face_ids = faces.cpu()
-        self.all_nodes = vertices[:n_vert.value].cpu()
+        # the reference's node table: shared ids from the replayed pointers, unused ids squeezed out (:750-771)
+        self._topo.sync()
+        faces, vertices, _ = self._topo.final()
+        assert faces.shape[0] == len(leaf_order), "host topology and device cell state disagree on the leaf cells"
+        self.face_ids = pt.from_numpy(faces)
+        self.all_nodes = pt.from_numpy(vertices)
         self.all_centers = self._center[order_d].cpu()
         self.all_levels = self._level[order_d].to(pt.int64).cpu().unsqueeze(-1)
-        # device-resident copies for the export stage (not part of the reference's attribute set)
+        self._topo = None                                     # native handle: not part of the pickled object
         self._times["t_end_renumber"] = time()
 
     def _create_mesh_info(self, counter: int) -> None:

@@ -22,11 +22,7 @@ class SparseSpatialSampling:
                  save_name: str, grid_name: str = "grid_s_cube", uniform_levels: int = 5,
                  n_cells_max: Union[int, float] = None, min_metric: float = 0.75, max_delta_level: bool = False,
                  n_cells_iter_start: int = None, n_cells_iter_end: int = None, n_jobs: int = 1,
-                 relTol: Union[int, float] = 1e-3, reach_at_least: float = 0.75, pre_select_cells: bool = False,
-                 exact_topology: bool = True):
-        # exact_topology (not in the reference): True replays the reference's neighbour pointers / node ids on the host,
-        # so vertices, faces and the max_delta_level closure equal the reference's; False builds the vertex table on the
-        # device from the cell lattice (same cells, different vertex numbering)
+                 relTol: Union[int, float] = 1e-3, reach_at_least: float = 0.75, pre_select_cells: bool = False):
         self.n_jobs = n_jobs
         self.coordinates = coordinates
         self.metric = metric
@@ -59,7 +55,7 @@ class SparseSpatialSampling:
                                       max_delta_level=self._max_delta_level, n_cells_iter_end=self._n_cells_iter_end,
                                       n_cells_iter_start=self._n_cells_iter_start, n_jobs=self.n_jobs,
                                       relTol=self._relTol, reach_at_least=self._reach_at_least,
-                                      pre_select=self._pre_select_cells, exact_topology=exact_topology)
+                                      pre_select=self._pre_select_cells)
 
     def execute_grid_generation(self) -> None:
         """Run S^3; afterwards ``centers, vertices, faces, levels, size_initial_cell`` are set (CPU tensors) and

@@ -2,8 +2,8 @@
 GPU parity of the refinement engine (SamplingTree.refine, s_cube.py:563-667):
   * against golden outputs of the REFERENCE itself (tests/golden/*.npz, made by tests/golden/make_golden.py),
   * against the CPU oracle on inputs that are not in the fixtures.
-Bit-exact: leaf cells (centre bits, level, numbering), N_leaf per iteration, gains and metrics of the leaves, and -- with
-the host-side pointer replay (default) -- the vertex table and the faces (node numbering) of the reference.
+Bit-exact: leaf cells (centre bits, level, numbering), N_leaf per iteration, gains and metrics of the leaves, and -- from
+the host-side pointer replay -- the vertex table and the faces (node numbering) of the reference.
 Tolerance: metric_per_iter 1e-12 relative (the reference reduces the norm with torch, a different summation tree).
 """
 import os
@@ -20,10 +20,10 @@ pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
-def _run(case, **extra):
+def _run(case):
     import sparsespatialsampling_b200.geometry as geo
     from sparsespatialsampling_b200.s_cube import SamplingTree
-    tree = SamplingTree(case["coords"], case["metric"], case["geoms"](geo), **case["kwargs"], sdm_order=1, **extra)
+    tree = SamplingTree(case["coords"], case["metric"], case["geoms"](geo), **case["kwargs"], sdm_order=1)
     tree.refine()
     return tree
 
@@ -54,24 +54,6 @@ def test_refine_matches_reference_golden(cuda, name):
     assert tree.face_ids.dtype == pt.int32
     assert np.array_equal(tree.face_ids.numpy(), ref["faces"])
     assert np.array_equal(tree.all_nodes.numpy(), ref["vertices"])
-
-
-@pytest.mark.parametrize("name", ["g2d_metric", "g3d_metric"])
-def test_lattice_vertex_table_variant(cuda, name):
-    # exact_topology=False: vertices from a lattice de-duplication on the device -- same cells, per-cell corner
-    # coordinates within 1e-12 * width of the reference's, different vertex numbering
-    import sparsespatialsampling_b200.geometry as geo
-    case = case_definitions(geo)[name]
-    ref = np.load(os.path.join(GOLDEN, f"{name}.npz"))
-    tree = _run(case, exact_topology=False)
-    assert list(tree._leaf_cells) == ref["leaf_index"].tolist()
-    assert np.array_equal(tree.all_centers.numpy(), ref["centers"])
-    mine = tree.all_nodes.numpy()[tree.face_ids.numpy().astype(np.int64)]
-    theirs = ref["vertices"][ref["faces"].astype(np.int64)]
-    assert mine.shape == theirs.shape
-    assert np.abs(mine - theirs).max() <= 1e-12 * float(ref["width"])
-    # every vertex is used, no duplicate coordinates in the table
-    assert np.unique(tree.face_ids.numpy()).size == tree.all_nodes.shape[0]
 
 
 @pytest.mark.parametrize("name", ["g2d_metric", "g3d_metric"])
