@@ -130,6 +130,7 @@ class SamplingTree(object):
         # pinned staging of the per-iteration transfers: parent list up, (invalid flags, captured-metric sum) down with
         # ONE synchronisation per iteration
         self._pin_i64 = pt.empty(1024, dtype=pt.int64, pin_memory=True)
+        self._pin_i64_copied = pt.cuda.Event()      # recorded behind the last host-to-device copy out of _pin_i64
         self._pin_u8 = pt.empty(8192, dtype=pt.uint8, pin_memory=True)
         self._pin_f64 = pt.empty(1, dtype=pt.float64, pin_memory=True)
         self._pin_sel = pt.empty(1024, dtype=pt.int64, pin_memory=True)
@@ -256,8 +257,12 @@ class SamplingTree(object):
         par_h = np.asarray(parents, dtype=np.int64)
         if n_par > self._pin_i64.numel():
             self._pin_i64 = pt.empty(2 * n_par, dtype=pt.int64, pin_memory=True)
-        self._pin_i64[:n_par].numpy()[:] = par_h         # (the previous iteration's copy was synchronised)
+        # the previous copy out of the pinned buffer may still be queued: the mask pass synchronises the stream after
+        # every refinement step, but with pre_select nothing does between two uniform levels
+        self._pin_i64_copied.synchronize()
+        self._pin_i64[:n_par].numpy()[:] = par_h
         par_d = self._pin_i64[:n_par].to(self._device, non_blocking=True)
+        self._pin_i64_copied.record(self._stream_obj or pt.cuda.current_stream(self._device))
         if self._stream_obj is None:
             pt.cuda.set_device(self._device)
         _lib.check(self._lib.s3_cells_refine(self._p("_center"), self._p("_level"), self._p("_flags"), _lib.ptr(par_d),
