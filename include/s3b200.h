@@ -232,6 +232,21 @@ int s3_svd_project(const float* d_a, const float* d_mean, const float* d_vs, int
 int s3_svd_project_tc(const float* d_a, const float* d_mean, const float* d_vol, int vol_div, const float* d_vs,
                       int64_t m, int64_t t, int r, int method, float* d_u, void* stream);
 
+/* ---- residual of a low-rank model (DMD / truncated POD reconstruction error) ------------------------
+ * e[m, t] = (a[m, t] - mean[m]) - sum_j left[m, j] * right_t[t, j]
+ * a fp32 [m, t] dense row-major (vector fields stacked as in s3_svd_gram, one vol per vol_div rows);
+ * d_mean fp32 [m] or NULL (= 0); d_vol fp32 [m / vol_div] or NULL (= 1); left fp32 [m, q]; right_t fp32 [t, q];
+ * 1 <= q <= 512 (larger q: S3_ERR_UNSUPPORTED). The product runs on tcgen05 (3xTF32), e is formed in fp64 and `a` is
+ * read once. Outputs, component c = m % vol_div:
+ *   d_sq_err  fp64 [vol_div, t] = sum_m vol * e^2
+ *   d_sq_ref  fp64 [vol_div, t] = sum_m vol * (a - mean)^2
+ *   d_max_abs fp64 [vol_div, t] = max_m |e|
+ *   d_row_sq_err fp64 [m] or NULL: sum_t e^2 ADDED into row m
+ * Every sum is reduced in a fixed order that depends on m and t only: bit-identical from run to run.        */
+int s3_lowrank_error(const float* d_a, int64_t m, int64_t t, const float* d_mean, const float* d_vol, int vol_div,
+                     const float* d_left, const float* d_right_t, int q, double* d_sq_err, double* d_sq_ref,
+                     double* d_max_abs, double* d_row_sq_err, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -16,7 +16,8 @@ from .export import ExportData, Fields
 from .data import Datawriter, Dataloader, XDMFWriter
 from .svd import compute_svd, compute_svd_sharded
 from .reconstruction import ReconstructionError, ErrorStats
-from .utils import write_svd_s_cube_to_file, export_fields_batchwise, export_openfoam_fields
+from .dmd import compute_dmd, DMD
+from .utils import write_svd_s_cube_to_file, write_dmd_s_cube_to_file, export_fields_batchwise, export_openfoam_fields
 from . import geometry
 
 _logging.getLogger(__name__).addHandler(_logging.NullHandler())
@@ -24,5 +25,5 @@ _logging.getLogger(__name__).addHandler(_logging.NullHandler())
 __version__ = "0.1.0"
 __all__ = ["SparseSpatialSampling", "SamplingTree", "list_geometries", "interpolate_data", "interp_gather", "KnnIndex",
            "ExportData", "Fields", "Datawriter", "Dataloader", "XDMFWriter", "compute_svd", "compute_svd_sharded", "ReconstructionError", "ErrorStats",
-           "write_svd_s_cube_to_file", "export_fields_batchwise", "export_openfoam_fields",
+           "compute_dmd", "DMD", "write_svd_s_cube_to_file", "write_dmd_s_cube_to_file", "export_fields_batchwise", "export_openfoam_fields",
            "geometry"]

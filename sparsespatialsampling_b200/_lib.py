@@ -74,6 +74,8 @@ _SIGNATURES = {
     "s3_svd_project": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p, c_void_p]),
     "s3_svd_project_tc": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_int64, c_int, c_int,
                                   c_void_p, c_void_p]),
+    "s3_lowrank_error": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int,
+                                 c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 

@@ -82,7 +82,7 @@ int s3_gather_rows(const float* src, int64_t src_pitch, const int32_t* d_rows, i
 
 const char* s3_last_error(void) { return s3::g_error; }
 
-int s3_version(void) { return 101; }
+int s3_version(void) { return 102; }
 
 int64_t s3_launch_count(void) { return s3::g_launches.load(std::memory_order_relaxed); }
 

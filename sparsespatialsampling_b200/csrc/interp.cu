@@ -43,6 +43,7 @@ extern int g_tc_seg_kblocks;
 extern int g_tc_flush_segments;
 extern int g_tc_pair;
 extern int g_plane_rows_cap;       // key 17 (csrc/svd.cu): rows per TF32 plane chunk of the Gram / projection kernels, 0 = no cap
+extern int g_lowrank_cap;          // key 19 (csrc/svd.cu): CTAs of s3_lowrank_error at most, 0 = one per SM
 extern int g_curve;          // csrc/knn.cu: 0 = Morton, 1 = Hilbert order of the KNN index and of the processing order (key 30)
 
 template <typename T, int V>
@@ -767,6 +768,7 @@ extern "C" int s3x_tune(int key, int value) {
         case 14: S3_REQUIRE(value == 0 || value == 1, "s3x_tune: paired Gram kernel must be 0 or 1"); g_tc_pair = value; return S3_OK;
         case 17: S3_REQUIRE(value >= 0, "s3x_tune: plane-row cap must be 0 (none) or >= 1"); g_plane_rows_cap = value; return S3_OK;
         case 18: S3_REQUIRE(value >= 0, "s3x_tune: reconstruction-error CTA cap must be 0 (none) or >= 1"); g_recon_cap = value; return S3_OK;
+        case 19: S3_REQUIRE(value >= 0, "s3x_tune: low-rank error CTA cap must be 0 (none) or >= 1"); g_lowrank_cap = value; return S3_OK;
     }
     s3::set_error("s3x_tune: unknown key %d", key);
     return S3_ERR_INVALID;

@@ -760,6 +760,292 @@ project_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
     }
 }
 
+// ================================================================== residual of a low-rank model (s3_lowrank_error)
+//   e[m][t] = (a[m][t] - mean[m]) - sum_j left[m][j] * right_t[t][j],   j < q <= 512
+// The product runs on tcgen05 with the operand forms of project_tc_kernel: left (K = q contiguous) takes the role of the
+// planes, right_t the role of W^T; both are split into TF32 hi / lo planes ([rows_pad][q_pad], zero padded) by
+// lowrank_prepare_kernel and contracted 3xTF32 into one 128 x 256 fp32 tile in TMEM (q_pad / 8 * 3 <= 192 MMAs, one
+// segment). The epilogue warps pull the tile with tcgen05.ld, read the matching 128 x 256 tile of `a` from HBM once and
+// form e in fp64. Work unit: a row tile (128 rows) over ALL column tiles, so that the row sums stay in registers of one
+// CTA; row tiles are dealt out in fixed groups of consecutive tiles (the grouping depends on m only), a group's column
+// partials are added up by one thread per column in tile order, and a second kernel sums the groups in group order:
+// the results do not depend on the number of CTAs. Accumulator double-buffered in TMEM (2 x 256 columns), so the MMAs of
+// the next column tile run under the epilogue of this one. Warp 0 = TMA, warp 1 = MMA, warps 2..5 = epilogue (one per
+// TMEM lane quarter; with eight, the register budget of 10 warps per SM spilled the fp64 reductions).
+constexpr int kLrBM = 128, kLrBN = 256, kLrMaxQ = 512;
+constexpr int kLrStages = 2;
+constexpr int kLrABytes = kLrBM * 128;                       // 128 rows x 32 floats
+constexpr int kLrBBytes = kLrBN * 128;                       // 256 rows x 32 floats
+constexpr int kLrStageBytes = 2 * (kLrABytes + kLrBBytes);   // [A_hi][A_lo][B_hi][B_lo] = 96 KB
+constexpr int kLrEpiWarps = 4;                               // one per TMEM lane quarter (6 warps: up to 255 registers)
+constexpr int kLrThreads = (2 + kLrEpiWarps) * 32;
+constexpr int kLrTmemCols = 2 * kLrBN;
+constexpr size_t kLrSmemBytes = (size_t)kLrStages * kLrStageBytes + 1024;
+constexpr int kLrMaxGroups = 1024;                           // row-tile groups at most (scratch: groups x 3 x vol_div x t)
+int g_lowrank_cap = 0;                                       // CTAs at most (s3x_tune key 19; tests), 0 = one per SM
+
+// hi / lo TF32 planes of src [rows, q] -> [rows_pad, q_pad], zero beyond rows / q
+__global__ void __launch_bounds__(256)
+lowrank_prepare_kernel(const float* __restrict__ src, int64_t rows, int q, int64_t rows_pad, int q_pad,
+                       float* __restrict__ hi, float* __restrict__ lo) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= rows_pad * q_pad) return;
+    const int64_t r = e / q_pad;
+    const int j = (int)(e % q_pad);
+    const float v = (r < rows && j < q) ? src[r * q + j] : 0.f;
+    uint32_t hbits;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hbits) : "f"(v));
+    const float h = __uint_as_float(hbits);
+    hi[e] = h;
+    lo[e] = v - h;
+}
+
+// Sum over the 32 lanes of a warp of each of 32 columns, value(j) = this lane's entry of column j (reduce-scatter
+// butterfly, 31 shuffles): returns the sum (max: the maximum) of column `lane`. The order of the adds is fixed by the lane
+// numbers. The first step consumes the values as they are formed, so only 16 partials are ever live.
+template <typename F>
+__device__ __forceinline__ double warp_column_reduce(F value, bool max, int lane) {
+    double v[16];
+    {
+        const bool upper = (lane & 16) != 0;
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+            const double lo = value(i), hi = value(i + 16);
+            const double recv = shfl_xor_d(upper ? lo : hi, 16);
+            v[i] = max ? fmax(upper ? hi : lo, recv) : (upper ? hi : lo) + recv;
+        }
+    }
+#pragma unroll
+    for (int k = 8; k >= 1; k >>= 1) {
+        const bool upper = (lane & k) != 0;
+#pragma unroll
+        for (int i = 0; i < k; ++i) {
+            const double send = upper ? v[i] : v[i + k];
+            const double keep = upper ? v[i + k] : v[i];
+            const double recv = shfl_xor_d(send, k);
+            v[i] = max ? fmax(keep, recv) : keep + recv;
+        }
+    }
+    return v[0];
+}
+
+__device__ __forceinline__ void named_bar(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
+
+// part: fp64 [n_groups][3][vol_div][t] (sq_err, sq_ref, max_abs of the group's rows)
+__global__ void __launch_bounds__(kLrThreads, 1)
+lowrank_error_kernel(const __grid_constant__ CUtensorMap map_lhi, const __grid_constant__ CUtensorMap map_llo,
+                     const __grid_constant__ CUtensorMap map_rhi, const __grid_constant__ CUtensorMap map_rlo,
+                     const float* __restrict__ a, const float* __restrict__ mean, const float* __restrict__ vol,
+                     int vol_div, int64_t m, int64_t t, int n_kgroups, int n_ct, int64_t n_rt, int64_t tiles_per_group,
+                     int64_t n_groups, double* __restrict__ part, double* __restrict__ row_sq_err) {
+    extern __shared__ __align__(1024) unsigned char lr_smem_raw[];
+    __shared__ __align__(8) uint64_t full_bar[kLrStages];
+    __shared__ __align__(8) uint64_t empty_bar[kLrStages];
+    __shared__ __align__(8) uint64_t acc_full_bar[2];
+    __shared__ __align__(8) uint64_t acc_empty_bar[2];
+    __shared__ uint32_t tmem_base_slot;
+    __shared__ double red[4][3][32];                         // [lane quarter][quantity][column]
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t raw = smem_u32(lr_smem_raw);
+    const uint32_t ring = (raw + 1023u) & ~1023u;
+    unsigned char* ring_ptr = lr_smem_raw + (ring - raw);
+
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < kLrStages; ++s) {
+            mbar_init(&full_bar[s], 1);
+            mbar_init(&empty_bar[s], 1);
+        }
+        for (int b = 0; b < 2; ++b) {
+            mbar_init(&acc_full_bar[b], 1);
+            mbar_init(&acc_empty_bar[b], kLrEpiWarps * 32);
+        }
+        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_lhi) : "memory");
+        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_rhi) : "memory");
+    }
+    if (warp == 1) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)),
+                     "r"((uint32_t)kLrTmemCols)
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = tmem_base_slot;
+
+    if (warp == 0) {
+        if (lane == 0) {
+            int it = 0;
+            for (int64_t grp = blockIdx.x; grp < n_groups; grp += gridDim.x) {
+                const int64_t rt1 = (grp + 1) * tiles_per_group < n_rt ? (grp + 1) * tiles_per_group : n_rt;
+                for (int64_t rt = grp * tiles_per_group; rt < rt1; ++rt)
+                    for (int ct = 0; ct < n_ct; ++ct)
+                        for (int g = 0; g < n_kgroups; ++g, ++it) {
+                            const int s = it % kLrStages;
+                            const uint32_t round = (uint32_t)(it / kLrStages);
+                            if (round > 0) mbar_wait_wd(&empty_bar[s], (round - 1) & 1u);
+                            unsigned char* st = ring_ptr + (size_t)s * kLrStageBytes;
+                            mbar_expect_tx(&full_bar[s], (uint32_t)kLrStageBytes);
+                            tma_load_2d(st, &map_lhi, g * 32, (int)(rt * kLrBM), &full_bar[s]);
+                            tma_load_2d(st + kLrABytes, &map_llo, g * 32, (int)(rt * kLrBM), &full_bar[s]);
+                            tma_load_2d(st + 2 * kLrABytes, &map_rhi, g * 32, ct * kLrBN, &full_bar[s]);
+                            tma_load_2d(st + 2 * kLrABytes + kLrBBytes, &map_rlo, g * 32, ct * kLrBN, &full_bar[s]);
+                        }
+            }
+        }
+        __syncwarp();
+    } else if (warp == 1) {
+        if (lane == 0) {
+            constexpr uint32_t idesc = umma_idesc_tf32_k(kLrBM, kLrBN);
+            int it = 0, item = 0;
+            for (int64_t grp = blockIdx.x; grp < n_groups; grp += gridDim.x) {
+                const int64_t rt1 = (grp + 1) * tiles_per_group < n_rt ? (grp + 1) * tiles_per_group : n_rt;
+                for (int64_t rt = grp * tiles_per_group; rt < rt1; ++rt)
+                    for (int ct = 0; ct < n_ct; ++ct, ++item) {
+                        const int b = item & 1;
+                        if (item >= 2) {
+                            mbar_wait_wd(&acc_empty_bar[b], (uint32_t)((item >> 1) - 1) & 1u);
+                            tc_fence_after();
+                        }
+                        const uint32_t d_tmem = tmem_base + (uint32_t)(b * kLrBN);
+                        uint32_t accumulate = 0;
+                        for (int g = 0; g < n_kgroups; ++g, ++it) {
+                            const int s = it % kLrStages;
+                            mbar_wait_wd(&full_bar[s], (uint32_t)(it / kLrStages) & 1u);
+                            tc_fence_after();
+                            const uint32_t st = ring + (uint32_t)s * kLrStageBytes;
+#pragma unroll
+                            for (int ks = 0; ks < 4; ++ks) {
+                                const uint32_t koff = (uint32_t)ks * 32u;
+                                const uint64_t a_hi = umma_desc_k_sw128(st + koff);
+                                const uint64_t a_lo = umma_desc_k_sw128(st + kLrABytes + koff);
+                                const uint64_t b_hi = umma_desc_k_sw128(st + 2 * kLrABytes + koff);
+                                const uint64_t b_lo = umma_desc_k_sw128(st + 2 * kLrABytes + kLrBBytes + koff);
+                                umma_tf32(d_tmem, a_lo, b_hi, idesc, accumulate);
+                                umma_tf32(d_tmem, a_hi, b_lo, idesc, 1u);
+                                umma_tf32(d_tmem, a_hi, b_hi, idesc, 1u);
+                                accumulate = 1u;
+                            }
+                            umma_commit(&empty_bar[s]);
+                        }
+                        umma_commit(&acc_full_bar[b]);
+                    }
+            }
+        }
+        __syncwarp();
+    } else {
+        const int qd = warp & 3;                             // TMEM lane quarter
+        // 16-byte row loads when every row starts 16-byte aligned (a lane reads its own row: a quarter of the load
+        // instructions of the scalar path, each touching the same 32 rows)
+        const bool vec4 = t % 4 == 0 && (reinterpret_cast<uintptr_t>(a) & 15) == 0;
+        int item = 0;
+        for (int64_t grp = blockIdx.x; grp < n_groups; grp += gridDim.x) {
+            const int64_t rt0 = grp * tiles_per_group;
+            const int64_t rt1 = rt0 + tiles_per_group < n_rt ? rt0 + tiles_per_group : n_rt;
+            for (int64_t rt = rt0; rt < rt1; ++rt) {
+                const int64_t row = rt * kLrBM + qd * 32 + lane;
+                const bool live = row < m;
+                const double mu = (live && mean) ? (double)mean[row] : 0.0;
+                const double w = live ? (vol ? (double)vol[row / vol_div] : 1.0) : 0.0;
+                const int comp = (int)(row % vol_div);
+                const float* arow = a + (live ? row : 0) * t;
+                double row_acc = 0.0;
+                for (int ct = 0; ct < n_ct; ++ct, ++item) {
+                    const int b = item & 1;
+                    const uint32_t taddr = tmem_base + ((uint32_t)(qd * 32) << 16) + (uint32_t)(b * kLrBN);
+#pragma unroll 1
+                    for (int c0 = 0; c0 < kLrBN; c0 += 32) {
+                        const int64_t col0 = (int64_t)ct * kLrBN + c0;
+                        float av[32];
+                        if (vec4) {                                       // t % 4 == 0: a float4 is all in or all out
+#pragma unroll
+                            for (int j = 0; j < 32; j += 4) {
+                                const float4 v = (live && col0 + j < t) ? __ldg(reinterpret_cast<const float4*>(arow + col0 + j))
+                                                                        : make_float4(0.f, 0.f, 0.f, 0.f);
+                                av[j] = v.x; av[j + 1] = v.y; av[j + 2] = v.z; av[j + 3] = v.w;
+                            }
+                        } else {
+#pragma unroll
+                            for (int j = 0; j < 32; ++j) av[j] = (live && col0 + j < t) ? __ldg(arow + col0 + j) : 0.f;
+                        }
+                        if (c0 == 0) {                                    // (the first loads are in flight meanwhile)
+                            mbar_wait_wd(&acc_full_bar[b], (uint32_t)(item >> 1) & 1u);
+                            tc_fence_after();
+                        }
+                        uint32_t pv[32];
+                        tmem_ld32(taddr + (uint32_t)c0, pv);             // warp-collective: all lanes, also dead rows
+                        if (c0 + 32 == kLrBN) {                       // the whole buffer is in registers
+                            tc_fence_before();
+                            mbar_arrive_cta(&acc_empty_bar[b]);
+                        }
+                        // the residual is formed in fp64 (no cancellation between a - mean and the product) and kept
+                        // rounded to fp32 (6e-8 of itself) for the reductions, which square and sum it in fp64; an fp64
+                        // copy of the chunk does not fit beside the butterfly in 255 registers. 0 past column t.
+                        float e[32];
+#pragma unroll
+                        for (int j = 0; j < 32; ++j) {
+                            e[j] = col0 + j < t ? (float)(((double)av[j] - mu) - (double)__uint_as_float(pv[j])) : 0.f;
+                            row_acc = fma((double)e[j], (double)e[j], row_acc);
+                        }
+                        const bool first = rt == rt0;
+#pragma unroll 1
+                        for (int c = 0; c < vol_div; ++c) {
+                            const double wc = comp == c ? w : 0.0;
+                            const bool in_c = live && comp == c;
+                            // one quantity at a time (k = 0: sum vol e^2, 1: sum vol (a - mean)^2, 2: max |e|): three
+                            // independent butterflies in flight at once would not fit the register budget
+#pragma unroll 1
+                            for (int k = 0; k < 3; ++k)
+                                red[qd][k][lane] = warp_column_reduce([&](int j) {
+                                    const double x = k == 1 ? (double)av[j] - mu : (double)e[j];
+                                    return k == 2 ? (in_c ? fabs(x) : 0.0) : wc * (x * x);
+                                }, k == 2, lane);
+                            named_bar(1, kLrEpiWarps * 32);
+                            // quarters 0..2 each combine one quantity over the four quarters, in order
+                            const int64_t col = col0 + lane;
+                            if (qd < 3 && col < t) {
+                                const double* r4 = &red[0][qd][lane];
+                                double sum;
+                                if (qd == 2) sum = fmax(fmax(r4[0], r4[3 * 32]), fmax(r4[6 * 32], r4[9 * 32]));
+                                else sum = ((r4[0] + r4[3 * 32]) + r4[6 * 32]) + r4[9 * 32];
+                                double* o = part + ((grp * 3 + qd) * vol_div + c) * t + col;
+                                if (!first) sum = qd == 2 ? fmax(*o, sum) : *o + sum;
+                                *o = sum;
+                            }
+                            named_bar(1, kLrEpiWarps * 32);
+                        }
+                    }
+                }
+                if (row_sq_err && live) row_sq_err[row] += row_acc;
+            }
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) {
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)kLrTmemCols)
+                     : "memory");
+    }
+}
+
+// out[k][c][col] = sum (k = 0, 1) / max (k = 2) over the groups, in group order; part [n_groups][3][vol_div][t]
+__global__ void __launch_bounds__(256)
+lowrank_reduce_kernel(const double* __restrict__ part, int64_t n_groups, int vol_div, int64_t t,
+                      double* __restrict__ sq_err, double* __restrict__ sq_ref, double* __restrict__ max_abs) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t n = 3 * (int64_t)vol_div * t;
+    if (e >= n) return;
+    const int k = (int)(e / ((int64_t)vol_div * t));
+    double acc = 0.0;
+    for (int64_t g = 0; g < n_groups; ++g) {
+        const double v = part[g * n + e];
+        acc = k == 2 ? fmax(acc, v) : acc + v;
+    }
+    const int64_t o = e % ((int64_t)vol_div * t);
+    (k == 0 ? sq_err : k == 1 ? sq_ref : max_abs)[o] = acc;
+}
+
 }  // namespace s3
 
 using namespace s3;
@@ -1029,4 +1315,76 @@ extern "C" int s3_svd_project_tc(const float* d_a, const float* d_mean, const fl
     S3_REQUIRE(method == 1 || method == 2, "s3_svd_project_tc: method must be 1 (3xTF32) or 2 (TF32)");
     if (m == 0) return S3_OK;
     return project_tc(d_a, d_mean, d_vol, vol_div, d_vs, m, t, r, method == 1 ? 3 : 1, d_u, (cudaStream_t)stream);
+}
+
+// e = (a - mean) - left right_t^T on the tensor cores with fused fp64 reductions (see lowrank_error_kernel)
+extern "C" int s3_lowrank_error(const float* d_a, int64_t m, int64_t t, const float* d_mean, const float* d_vol,
+                                int vol_div, const float* d_left, const float* d_right_t, int q, double* d_sq_err,
+                                double* d_sq_ref, double* d_max_abs, double* d_row_sq_err, void* stream) {
+    S3_REQUIRE(d_a && d_left && d_right_t, "s3_lowrank_error: NULL argument");
+    S3_REQUIRE(d_sq_err && d_sq_ref && d_max_abs, "s3_lowrank_error: NULL result");
+    S3_REQUIRE(m >= 1 && t >= 1 && vol_div >= 1, "s3_lowrank_error: bad sizes (m %lld, t %lld, vol_div %d)",
+               (long long)m, (long long)t, vol_div);
+    S3_REQUIRE(m % vol_div == 0, "s3_lowrank_error: m = %lld rows is not a multiple of vol_div = %d", (long long)m,
+               vol_div);
+    S3_REQUIRE(m <= ((int64_t)1 << 31) - kLrBM && t <= ((int64_t)1 << 31) - kLrBN,
+               "s3_lowrank_error: too many rows or columns (%lld x %lld)", (long long)m, (long long)t);
+    if (q < 1 || q > kLrMaxQ) {
+        s3::set_error("s3_lowrank_error: q = %d columns of left / right_t, supported 1..%d (one 3xTF32 TMEM segment)", q,
+                      kLrMaxQ);
+        return S3_ERR_UNSUPPORTED;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    static PFN_encodeTiledSvd encode = nullptr;
+    if (!encode) {
+        void* fn = nullptr;
+        cudaDriverEntryPointQueryResult qres;
+        S3_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
+        S3_REQUIRE(fn != nullptr && qres == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled not available");
+        encode = (PFN_encodeTiledSvd)fn;
+    }
+    const int q_pad = (int)(ceil_div((int64_t)q, (int64_t)32) * 32);
+    const int64_t m_pad = ceil_div(m, (int64_t)kLrBM) * kLrBM, t_pad = ceil_div(t, (int64_t)kLrBN) * kLrBN;
+    const int64_t n_rt = m_pad / kLrBM;
+    const int n_ct = (int)(t_pad / kLrBN);
+    // row tiles per group: a function of m only, so that the sums do not depend on the CTA count
+    const int64_t tiles_per_group = ceil_div(n_rt, (int64_t)kLrMaxGroups);
+    const int64_t n_groups = ceil_div(n_rt, tiles_per_group);
+    int64_t ctas = n_groups < kNumSMs ? n_groups : kNumSMs;
+    if (g_lowrank_cap > 0 && ctas > g_lowrank_cap) ctas = g_lowrank_cap;
+
+    Scratch scratch(st);
+    float *lhi = nullptr, *llo = nullptr, *rhi = nullptr, *rlo = nullptr;
+    double* part = nullptr;
+    S3_TRY(scratch.alloc(&lhi, (size_t)m_pad * q_pad));
+    S3_TRY(scratch.alloc(&llo, (size_t)m_pad * q_pad));
+    S3_TRY(scratch.alloc(&rhi, (size_t)t_pad * q_pad));
+    S3_TRY(scratch.alloc(&rlo, (size_t)t_pad * q_pad));
+    S3_TRY(scratch.alloc(&part, (size_t)n_groups * 3 * vol_div * t));
+    lowrank_prepare_kernel<<<(unsigned)ceil_div(m_pad * q_pad, (int64_t)256), 256, 0, st>>>(d_left, m, q, m_pad, q_pad,
+                                                                                          lhi, llo);
+    lowrank_prepare_kernel<<<(unsigned)ceil_div(t_pad * q_pad, (int64_t)256), 256, 0, st>>>(d_right_t, t, q, t_pad,
+                                                                                          q_pad, rhi, rlo);
+    CUtensorMap maps[4];
+    float* planes[4] = {lhi, llo, rhi, rlo};
+    for (int i = 0; i < 4; ++i) {
+        memset(&maps[i], 0, sizeof(CUtensorMap));
+        const cuuint64_t gdim[2] = {(cuuint64_t)q_pad, (cuuint64_t)(i < 2 ? m_pad : t_pad)};
+        const cuuint64_t gstride[1] = {(cuuint64_t)q_pad * 4};
+        const cuuint32_t box[2] = {32, (cuuint32_t)(i < 2 ? kLrBM : kLrBN)};
+        const cuuint32_t estride[2] = {1, 1};
+        CUresult cr = encode(&maps[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, planes[i], gdim, gstride, box, estride,
+                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        S3_REQUIRE(cr == CUDA_SUCCESS, "cuTensorMapEncodeTiled(low-rank plane %d) failed with code %d", i, (int)cr);
+    }
+    S3_CUDA(cudaFuncSetAttribute(lowrank_error_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrSmemBytes));
+    lowrank_error_kernel<<<(unsigned)ctas, kLrThreads, kLrSmemBytes, st>>>(
+        maps[0], maps[1], maps[2], maps[3], d_a, d_mean, d_vol, vol_div, m, t, q_pad / 32, n_ct, n_rt, tiles_per_group,
+        n_groups, part, d_row_sq_err);
+    lowrank_reduce_kernel<<<(unsigned)ceil_div(3 * (int64_t)vol_div * t, (int64_t)256), 256, 0, st>>>(
+        part, n_groups, vol_div, t, d_sq_err, d_sq_ref, d_max_abs);
+    S3_LAUNCH_CHECK();
+    note_launch(4);
+    return S3_OK;
 }

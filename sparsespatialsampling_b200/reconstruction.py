@@ -51,7 +51,9 @@ class ErrorStats:
 
     ``sq_err`` / ``sq_ref`` / ``max_abs`` ``[D, T_seen]``: per component and snapshot, the sum over the original points
     of ``e^2`` and of ``original^2``, and the largest ``|e|``; ``point_sq_err`` ``[N, D]``: per original point (order of
-    ``coordinates``) and component, the sum of ``e^2`` over the snapshots; ``n_snapshots`` = ``T_seen``."""
+    ``coordinates``) and component, the sum of ``e^2`` over the snapshots; ``n_snapshots`` = ``T_seen``. For errors on
+    the grid side (``DMD.reconstruction_error``, ``svd.reconstruction_error``) ``sq_err`` / ``sq_ref`` are area-weighted
+    and ``point_sq_err`` is per cell."""
 
     def __init__(self, n_points: int, n_comp: int, device, distributed: bool = False, group=None):
         self.sq_err = pt.zeros((n_comp, 0), dtype=pt.float64, device=device)

@@ -51,6 +51,23 @@ def _as_device_matrix(data_matrix: pt.Tensor, dev) -> pt.Tensor:
     return a.contiguous()
 
 
+def _field_on_device(data_matrix: pt.Tensor, cell_area: pt.Tensor, device):
+    """Checks a ``[N_cells, T]`` / ``[N_cells, D, T]`` field and its cell areas and puts both on the compute device
+    (``device``, else the field's CUDA device, else the current one): ``(a [N_cells * D, T] fp32, vol [N_cells] fp32,
+    vol_div = D, compute device)``."""
+    shape = tuple(data_matrix.shape)
+    if len(shape) not in (2, 3):
+        raise ValueError(f"data_matrix must be [N_cells, T] or [N_cells, D, T], got {shape}")
+    if cell_area.numel() != shape[0]:
+        raise ValueError(f"cell_area has {cell_area.numel()} entries for {shape[0]} cells")
+    home = data_matrix.device
+    dev = pt.device(device) if device is not None else (home if home.type == "cuda" else pt.device("cuda", pt.cuda.current_device()))
+    vol_div = 1 if len(shape) == 2 else shape[1]
+    a = _as_device_matrix(data_matrix, dev).reshape(shape[0] * vol_div, shape[-1])
+    vol = cell_area.detach().reshape(-1).to(device=dev, dtype=pt.float32).contiguous()
+    return a, vol, vol_div, dev
+
+
 def row_means(a: pt.Tensor) -> pt.Tensor:
     """Temporal mean of every row of ``a`` ([M, T] fp32 on the device)."""
     lib = _lib.load()
@@ -99,6 +116,85 @@ def project_tc(a: pt.Tensor, mean: pt.Tensor, vol: pt.Tensor, vol_div: int, vs: 
     return u
 
 
+LOWRANK_MAX_Q = 512
+
+
+def lowrank_error(a: pt.Tensor, left: pt.Tensor, right_t: pt.Tensor, mean: pt.Tensor = None, vol: pt.Tensor = None,
+                  vol_div: int = 1, row_sq_err: pt.Tensor = None):
+    """Residual ``e = (a - mean[:, None]) - left @ right_t.T`` reduced without forming it (``s3_lowrank_error``: tcgen05
+    3xTF32 product, fp64 epilogue, ``a`` read once). ``a`` fp32 ``[M, T]``, ``left`` ``[M, q]``, ``right_t`` ``[T, q]``,
+    ``q <= 512``; ``mean`` ``[M]`` (``None`` = 0), ``vol`` ``[M / vol_div]`` (``None`` = 1). Returns ``(sq_err, sq_ref,
+    max_abs)`` fp64 ``[vol_div, T]`` (volume-weighted sums of ``e^2`` and ``(a - mean)^2``, largest ``|e|``, per
+    component ``m % vol_div``); ``sum_t e^2`` is added into ``row_sq_err`` fp64 ``[M]`` when it is given."""
+    lib = _lib.load()
+    for name, x in (("a", a), ("left", left), ("right_t", right_t), ("mean", mean), ("vol", vol)):
+        if x is not None and x.dtype != pt.float32:
+            raise ValueError(f"`{name}` must be float32, got {x.dtype}")
+    m, t = a.shape
+    if left.dim() != 2 or left.size(0) != m or right_t.dim() != 2 or right_t.size(0) != t or \
+            right_t.size(1) != left.size(1):
+        raise ValueError(f"left {tuple(left.shape)} / right_t {tuple(right_t.shape)} do not fit a {(m, t)} matrix")
+    if row_sq_err is not None and (row_sq_err.dtype != pt.float64 or row_sq_err.numel() != m):
+        raise ValueError("`row_sq_err` must be float64 with one entry per row")
+    if vol_div < 1 or m % vol_div:
+        raise ValueError(f"{m} rows are not a multiple of vol_div = {vol_div}")
+    if mean is not None and mean.numel() != m:
+        raise ValueError(f"`mean` has {mean.numel()} entries for {m} rows")
+    if vol is not None and vol.numel() != m // vol_div:
+        raise ValueError(f"`vol` has {vol.numel()} entries for {m // vol_div} cells ({m} rows / vol_div = {vol_div})")
+    for name, x in (("left", left), ("right_t", right_t), ("mean", mean), ("vol", vol), ("row_sq_err", row_sq_err)):
+        if x is not None and x.device != a.device:
+            raise ValueError(f"`{name}` is on {x.device}, `a` on {a.device}")
+    if a.device.type != "cuda":
+        raise ValueError(f"`a` must be a CUDA tensor, got {a.device}")
+    if row_sq_err is not None and not row_sq_err.is_contiguous():
+        raise ValueError("`row_sq_err` must be contiguous (the kernel adds into it)")
+    a, left, right_t = a.contiguous(), left.contiguous(), right_t.contiguous()
+    mean = mean.contiguous() if mean is not None else None
+    vol = vol.contiguous() if vol is not None else None
+    sq_err = pt.empty((vol_div, t), dtype=pt.float64, device=a.device)
+    sq_ref, max_abs = pt.empty_like(sq_err), pt.empty_like(sq_err)
+    with pt.cuda.device(a.device):
+        _lib.check(lib.s3_lowrank_error(_lib.ptr(a), m, t, _lib.ptr(mean), _lib.ptr(vol), vol_div, _lib.ptr(left),
+                                        _lib.ptr(right_t), left.size(1), _lib.ptr(sq_err), _lib.ptr(sq_ref),
+                                        _lib.ptr(max_abs), _lib.ptr(row_sq_err), _lib.stream_ptr()))
+    return sq_err, sq_ref, max_abs
+
+
+def _error_stats(a: pt.Tensor, left: pt.Tensor, right_t: pt.Tensor, mean, vol: pt.Tensor, vol_div: int):
+    """``ErrorStats`` of one low-rank model of the whole matrix ``a`` (rows = cells x components)."""
+    from .reconstruction import ErrorStats
+    n_cells = a.size(0) // vol_div
+    stats = ErrorStats(n_cells, vol_div, a.device)
+    row = pt.zeros((a.size(0),), dtype=pt.float64, device=a.device)
+    stats.sq_err, stats.sq_ref, stats.max_abs = lowrank_error(a, left, right_t, mean, vol, vol_div, row)
+    stats.point_sq_err = row.reshape(n_cells, vol_div)
+    stats.n_snapshots = a.size(1)
+    return stats
+
+
+def reconstruction_error(data_matrix: pt.Tensor, cell_area: pt.Tensor, s: pt.Tensor, U: pt.Tensor, V: pt.Tensor,
+                         device=None):
+    """
+    Truncation error of a POD model from ``compute_svd``: the field is rebuilt from the row means and the triplets the
+    caller passes (``s[:r]``, ``U[..., :r]``, ``V[:, :r]``), ``mean + U diag(s) V^T``, and compared with ``data_matrix``
+    (the same ``[N_cells, T]`` / ``[N_cells, D, T]`` input) by ``s3_lowrank_error`` without materialising it. Returns
+    ``ErrorStats``: area-weighted ``sq_err`` / ``sq_ref`` (``sq_ref`` = the centred field) and ``max_abs`` per component
+    and snapshot, ``point_sq_err`` per cell and component. ``r <= 512``.
+    """
+    _lib.require_cuda()
+    shape = tuple(data_matrix.shape)
+    r = int(s.numel())
+    if tuple(U.shape) != shape[:-1] + (r,) or tuple(V.shape) != (shape[-1], r):
+        raise ValueError(f"U {tuple(U.shape)} / V {tuple(V.shape)} do not match {r} singular values of a {shape} field")
+    if r > LOWRANK_MAX_Q:
+        raise ValueError(f"at most {LOWRANK_MAX_Q} modes, got {r}")
+    a, vol, vol_div, dev = _field_on_device(data_matrix, cell_area, device)
+    n_cells = shape[0]
+    left = (U.to(dev, pt.float64).reshape(n_cells * vol_div, r) * s.to(dev, pt.float64)[None, :]).float()
+    return _error_stats(a, left, V.to(dev, pt.float32), row_means(a), vol, vol_div)
+
+
 def compute_svd(data_matrix: pt.Tensor, cell_area: pt.Tensor, rank: int = None, method: str = "tc3",
                 n_modes: int = None, device=None) -> Tuple[pt.Tensor, pt.Tensor, pt.Tensor]:
     """
@@ -116,16 +212,9 @@ def compute_svd(data_matrix: pt.Tensor, cell_area: pt.Tensor, rank: int = None, 
     if method not in GRAM_METHODS:
         raise ValueError(f"unknown Gram method '{method}', available: {sorted(GRAM_METHODS)}")
     shape = tuple(data_matrix.shape)
-    if len(shape) not in (2, 3):
-        raise ValueError(f"data_matrix must be [N_cells, T] or [N_cells, D, T], got {shape}")
-    if cell_area.numel() != shape[0]:
-        raise ValueError(f"cell_area has {cell_area.numel()} entries for {shape[0]} cells")
     home = data_matrix.device
-    dev = pt.device(device) if device is not None else (home if home.type == "cuda" else pt.device("cuda", pt.cuda.current_device()))
-    n_cells, t = shape[0], shape[-1]
-    vol_div = 1 if len(shape) == 2 else shape[1]
-    a = _as_device_matrix(data_matrix, dev).reshape(n_cells * vol_div, t)
-    vol = cell_area.detach().reshape(-1).to(device=dev, dtype=pt.float32).contiguous()
+    a, vol, vol_div, dev = _field_on_device(data_matrix, cell_area, device)
+    n_cells = shape[0]
 
     mean = row_means(a)
     g = gram(a, mean, vol, vol_div, method)
@@ -205,20 +294,24 @@ def top_eigenpairs(g: pt.Tensor, r: int, tol: float = 1e-7, max_iter: int = 40):
     return None
 
 
+def eigenpairs(g: pt.Tensor, rank, r_max: int):
+    """Eigenpairs of the symmetric Gram matrix ``g`` in descending order: the top ``min(rank, r_max)`` by subspace
+    iteration when that converges (``EIG_METHOD = "auto"``, ``rank`` given), else all of them by ``torch.linalg.eigh``."""
+    top = None
+    if rank is not None and EIG_METHOD == "auto":
+        top = top_eigenpairs(g, max(1, min(int(rank), r_max)))
+    if top is not None:
+        return top                                     # descending, only the pairs that were asked for
+    lam, vec = pt.linalg.eigh(g)                       # ascending, fp64
+    return pt.flip(lam, dims=(0,)), pt.flip(vec, dims=(1,))
+
+
 def _factor(a: pt.Tensor, mean: pt.Tensor, g: pt.Tensor, rank, n_modes, rows_total: int, vol: pt.Tensor, vol_div: int,
             method: str):
     """Eigen-decomposition of the (summed) Gram matrix and projection of the rows held in ``a``."""
     t = a.size(1)
     r_max = min(rows_total, t)
-    top = None
-    if rank is not None and EIG_METHOD == "auto":
-        top = top_eigenpairs(g, max(1, min(int(rank), r_max)))
-    if top is not None:
-        lam, vec = top                                 # descending, only the pairs that were asked for
-    else:
-        lam, vec = pt.linalg.eigh(g)                   # ascending, fp64
-        lam = pt.flip(lam, dims=(0,))
-        vec = pt.flip(vec, dims=(1,))
+    lam, vec = eigenpairs(g, rank, r_max)
     s_all = lam.clamp_min(0.0).sqrt()
     if rank is None:
         r = optimal_rank(s_all[:r_max], rows_total, t)

@@ -1,6 +1,7 @@
 """
 Workflow helpers of the reference that sit on the accelerated path (sparseSpatialSampling/utils.py):
-``compute_svd`` (utils.py:302-346) and ``write_svd_s_cube_to_file`` (utils.py:349-413).
+``compute_svd`` (utils.py:302-346) and ``write_svd_s_cube_to_file`` (utils.py:349-413), and the DMD counterpart
+``write_dmd_s_cube_to_file``.
 
 The OpenFOAM loaders of the reference (``load_foam_data``, ``load_original_Foam_fields``, ``export_openfoam_fields``,
 utils.py:23-299) are file I/O through flowtorch and out of scope (SURVEY.md section 2).
@@ -9,11 +10,12 @@ import logging
 from typing import Union
 
 from .data import Dataloader, Datawriter
+from .dmd import compute_dmd
 from .svd import compute_svd
 
 logger = logging.getLogger(__name__)
 
-__all__ = ["compute_svd", "write_svd_s_cube_to_file"]
+__all__ = ["compute_svd", "write_svd_s_cube_to_file", "write_dmd_s_cube_to_file"]
 
 
 def write_svd_s_cube_to_file(field_names: Union[list, str], load_dir: str, file_name: str, new_file: bool,
@@ -52,6 +54,57 @@ def write_svd_s_cube_to_file(field_names: Union[list, str], load_dir: str, file_
         # not referenced by the XDMF file
         datawriter.write_data("V", group="constant", data=V)
         datawriter.write_data("s", group="constant", data=s)
+        datawriter.write_data("cell_area", group="constant", data=dataloader.weights)
+        datawriter.write_xdmf_file()
+
+
+def uniform_time_step(write_times) -> float:
+    """Spacing of ``write_times``; a spacing that varies by more than 1e-6 of itself raises ``ValueError``."""
+    times = sorted(float(t) for t in write_times)
+    if len(times) < 2:
+        raise ValueError(f"a time step needs at least 2 write times, got {len(times)}")
+    steps = [b - a for a, b in zip(times[:-1], times[1:])]
+    dt = (times[-1] - times[0]) / (len(times) - 1)
+    if dt <= 0 or max(abs(d - dt) for d in steps) > 1e-6 * dt:
+        raise ValueError(f"write times are not uniformly spaced (steps {min(steps)} .. {max(steps)}); pass dt")
+    return dt
+
+
+def write_dmd_s_cube_to_file(field_names: Union[list, str], load_dir: str, file_name: str, new_file: bool,
+                             dt: float = None, n_modes: int = None, rank=None, t_start: Union[int, float] = 0,
+                             method: str = "tc3") -> None:
+    """
+    DMD of exported fields (``compute_dmd``), written as ``<file_name>_<field>_dmd.h5`` (+ XDMF), arguments as
+    ``write_svd_s_cube_to_file``; ``dt = None`` takes the spacing of the write times. The file format has no complex
+    type, so ``constant`` holds real / imaginary pairs: ``mode_<i>_real`` / ``mode_<i>_imag`` (i = 1..n, ordered by
+    ``|amplitude|``), ``eigvals_real`` / ``eigvals_imag``, ``amplitude_real`` / ``amplitude_imag``, and ``frequency``,
+    ``growth_rate``, ``s``, ``cell_area``.
+    """
+    if type(field_names) is str:
+        field_names = [field_names]
+
+    for f in field_names:
+        logger.info(f"Performing DMD for field {f}.")
+        _name = f"{file_name}_{f}" if new_file else file_name
+        dataloader = Dataloader(load_dir, f"{_name}.h5")
+        _write_times = sorted([t for t in dataloader.write_times if float(t) >= t_start], key=lambda x: float(x))
+        step = uniform_time_step(_write_times) if dt is None else dt
+        dmd = compute_dmd(dataloader.load_snapshot(f, _write_times), dataloader.weights, step, rank=rank,
+                          n_modes=n_modes, method=method)
+
+        datawriter = Datawriter(load_dir, file_name + f"_{f}_dmd.h5")
+        datawriter.write_grid(dataloader)
+        modes = dmd.modes.cpu()
+        for i in range(dmd.n_modes):
+            datawriter.write_data(f"mode_{i + 1}_real", group="constant", data=modes[..., i].real.contiguous().squeeze())
+            datawriter.write_data(f"mode_{i + 1}_imag", group="constant", data=modes[..., i].imag.contiguous().squeeze())
+        for name in ("eigvals", "amplitude"):
+            value = getattr(dmd, name).cpu()
+            datawriter.write_data(f"{name}_real", group="constant", data=value.real.contiguous())
+            datawriter.write_data(f"{name}_imag", group="constant", data=value.imag.contiguous())
+        datawriter.write_data("frequency", group="constant", data=dmd.frequency.cpu())
+        datawriter.write_data("growth_rate", group="constant", data=dmd.growth_rate.cpu())
+        datawriter.write_data("s", group="constant", data=dmd.s.cpu())
         datawriter.write_data("cell_area", group="constant", data=dataloader.weights)
         datawriter.write_xdmf_file()
 
