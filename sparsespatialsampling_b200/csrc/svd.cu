@@ -4,9 +4,9 @@
 // eigen-decomposition is left to the host (torch.linalg.eigh, fp64).
 //
 // Gram contraction, 2*M*T^2 flop (the only GEMM-shaped work of the S^3 path, SURVEY 8a row a14):
-//   method 1/2 (default 1): tcgen05 tensor cores. A prepare kernel centres and scales the rows and writes them as
-//     TF32 "hi" (+ "lo" residual for the 3xTF32 split, method 1) planes in a [T/32][rows][32] layout; the Gram
-//     kernel is warp-specialised: one TMA producer thread (3-D boxes, 128B swizzle with 32B atoms, 4-stage mbarrier ring), one
+//   method 1/2 (default 1): tcgen05 tensor cores. gram_prepare_kernel centres and scales the rows and writes them as
+//     TF32 "hi" (+ "lo" residual for the 3xTF32 split, method 1) planes in a [T/32][rows][32] layout; gram_tc_kernel
+//     is warp-specialised: one TMA producer thread (3-D boxes, 128B swizzle with 32B atoms, 4-stage mbarrier ring), one
 //     thread issuing tcgen05.mma.kind::tf32 with both operands MN-major straight from the swizzled stages
 //     (D[128x256] += A_l*B_h + A_h*B_l + A_h*B_h), fp32 accumulators double-buffered in TMEM (2 x 256 columns),
 //     and eight epilogue warps that pull every finished K-segment (a few stages) out of TMEM with tcgen05.ld,
@@ -19,11 +19,11 @@
 //     by the tensor pipe + TMEM drains, not by operand traffic.
 //   method 0: fp32 CUDA-core tiles (kept as the on-device cross-check of the tensor-core path).
 // Projection U = (A - mean) V / s, 2*M*T*r flop: the same planes contracted over t on tcgen05 (project_tc_kernel, K-major
-//   TF32 operands, 3xTF32, a few TMEM segments against accumulation drift), 262144 x 2000 rows onto r = 50 / 150 / 256
-//   modes in 1.8 / 2.3 / 2.6 ms (of which 1.1 ms is the prepare pass) instead of 4.2 / 12.2 / 16.0 ms on the fp32
-//   CUDA-core kernel, max error vs fp64 2e-6 .. 8e-6 of the largest entry.
-#include <cuda.h>
-#include "common.cuh"
+//   TF32 operands, 3xTF32, a few TMEM segments against accumulation drift; tf32_split_kernel splits (V / s)^T),
+//   262144 x 2000 rows onto r = 50 / 150 / 256 modes in 1.8 / 2.3 / 2.6 ms (of which 1.1 ms is the prepare pass) instead
+//   of 4.2 / 12.2 / 16.0 ms on the fp32 CUDA-core kernel, max error vs fp64 2e-6 .. 8e-6 of the largest entry.
+// Residual of a low-rank model (s3_lowrank_error): lowrank_error_kernel, the operand forms of the projection with both
+//   factors split by tf32_split_kernel, and lowrank_reduce_kernel. The inline PTX of these kernels is in tma.cuh.
 #include "tma.cuh"
 #include "../../include/s3b200.h"
 
@@ -202,7 +202,7 @@ int g_plane_rows_cap = 0;       // rows per plane chunk of gram_tc / project_tc 
                                 // accumulation at small sizes), 0 = planes of up to 2 GB
 
 // Centre, scale and split the rows [row0, row0 + n_rows) of A into TF32 planes, layout [n_groups][plane_rows][32]:
-//   b = (a - mean) * sqrt(vol);  hi = tf32_rna(b);  lo = b - hi  (exact in fp32; the tensor core drops lo's low bits).
+//   b = (a - mean) * sqrt(vol);  (hi, lo) = tf32_split(b).
 // Rows past `m` and columns past `t` are written as zeros. One warp per row.
 __global__ void __launch_bounds__(256)
 gram_prepare_kernel(const float* __restrict__ a, const float* __restrict__ mean, const float* __restrict__ vol,
@@ -223,115 +223,27 @@ gram_prepare_kernel(const float* __restrict__ a, const float* __restrict__ mean,
         const int64_t c = (int64_t)g * 32 + lane;
         float b = 0.f;
         if (live && c < t) b = (p[c] - mu) * s;
-        uint32_t hbits;
-        asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hbits) : "f"(b));
-        const float h = __uint_as_float(hbits);
+        float h, l;
+        tf32_split(b, h, l);
         const int64_t o = ((int64_t)g * plane_rows + r) * 32 + lane;
         hi[o] = h;
-        if (lo) lo[o] = b - h;
+        if (lo) lo[o] = l;
     }
 }
 
-__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, int c0, int c1, int c2, uint64_t* bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::
-            "r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-// mbarrier wait with a watchdog: a protocol error must surface as a launch failure, not as a hung GPU
-__device__ __forceinline__ void mbar_wait_wd(uint64_t* bar, uint32_t phase) {
-    uint32_t done = 0;
-    const long long t0 = clock64();
-    while (true) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n"
-            : "=r"(done)
-            : "r"(smem_u32(bar)), "r"(phase)
-            : "memory");
-        if (done) break;
-        if (clock64() - t0 > 8000000000ll) __trap();
-    }
-}
-// the same box written to the same shared-memory offset of every CTA in `cta_mask`; each destination CTA's mbarrier at
-// the same offset receives the complete_tx for the bytes that landed in that CTA
-__device__ __forceinline__ void tma_load_3d_multicast(void* dst, const CUtensorMap* map, int c0, int c1, int c2,
-                                                      uint64_t* bar, uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-        " [%0], [%1, {%3, %4, %5}], [%2], %6;" ::"r"(smem_u32(dst)),
-        "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "h"(cta_mask)
-        : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_rank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cta(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// Shared-memory matrix descriptor of an MN-major TF32 operand. 32-bit MN-major operands have exactly one legal
-// swizzled layout, "128B swizzle with 32B atoms" (UMMA layout type 1; CUTLASS: Layout_MN_SW128_32B_Atom):
-//   (byte address) Swizzle<2,5,2> o ((32 floats, n), (4, k)) : ((4 B, LBO), (128 B, SBO))
-// i.e. 128-byte rows of 32 MN-contiguous floats, 4 K-rows per 512-byte atom, the 32-byte chunk index of a row is
-// XOR-ed with (row & 3); LBO = byte distance between 32-float MN groups, SBO = byte distance between 4-row K atoms.
-// This is what a TMA box {32 floats, rows, groups} written with CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B looks like.
-__device__ __forceinline__ uint64_t umma_desc_mn_sw128_32b(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    uint64_t d = 0;
-    d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);
-    d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16;
-    d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32;
-    d |= (uint64_t)1 << 46;     // descriptor version 1 (Blackwell)
-    d |= (uint64_t)1 << 61;     // layout type SWIZZLE_128B_BASE32B
-    return d;
-}
-// instruction descriptor: D fp32, A/B TF32, both MN-major ("transposed"), M x N
-__host__ __device__ constexpr uint32_t umma_idesc_tf32_mn(int M, int N) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(N >> 3) << 17) |
-           ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                          uint32_t accumulate) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
-        "}\n" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-                 : "memory");
-}
-// the same, arriving on the mbarrier at this offset in every CTA of `cta_mask`
-__device__ __forceinline__ void umma_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::
-                     "r"(smem_u32(bar)), "h"(cta_mask)
-                 : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-          "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-          "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-          "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+// TF32 planes [n_i_pad][n_c_pad] of a strided fp32 matrix: (hi, lo)[i][c] = tf32_split(src[i * s_i + c * s_c]) for
+// i < n_i, c < n_c, zeros in the padding; no lo plane when `lo` is NULL. The K-major operands W^T = (V / s)^T of the
+// projection and left / right_t of the low-rank residual.
+__global__ void __launch_bounds__(256)
+tf32_split_kernel(const float* __restrict__ src, int64_t s_i, int64_t s_c, int64_t n_i, int64_t n_c, int64_t n_i_pad,
+                  int64_t n_c_pad, float* __restrict__ hi, float* __restrict__ lo) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n_i_pad * n_c_pad) return;
+    const int64_t i = e / n_c_pad, c = e % n_c_pad;
+    float h, l;
+    tf32_split((i < n_i && c < n_c) ? src[i * s_i + c * s_c] : 0.f, h, l);
+    hi[e] = h;
+    if (lo) lo[e] = l;
 }
 
 // first j-tile (256 columns) that reaches the upper triangle of i-tile ti (128 rows)
@@ -406,15 +318,10 @@ gram_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant
             mbar_init(&acc_full_bar[b], 1);
             mbar_init(&acc_empty_bar[b], kTcEpiWarps * 32);
         }
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_hi) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_lo) : "memory");
+        tma_prefetch(&map_hi);
+        tma_prefetch(&map_lo);
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)),
-                     "r"((uint32_t)kTcTmemCols)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tmem_alloc(&tmem_base_slot, (uint32_t)kTcTmemCols);
     tc_fence_before();
     __syncthreads();
     if (PAIR) cluster_sync_all();                          // the peer's barriers exist before anything arrives on them
@@ -550,10 +457,7 @@ gram_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant
     tc_fence_before();
     __syncthreads();
     if (PAIR) cluster_sync_all();                          // the peer may still multicast into / arrive on this CTA
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)kTcTmemCols)
-                     : "memory");
-    }
+    if (warp == 1) tmem_dealloc(tmem_base, (uint32_t)kTcTmemCols);
 }
 
 // G[i][j] (+)= sum over splits of the tile partials; both triangles are written from the same upper-triangle entry.
@@ -596,44 +500,6 @@ constexpr int kPjABytes = kPjBM * 128;                       // one plane tile: 
 // measured 3.2e-5 / 5.1e-5 of the largest entry on a B200, split launches 7e-6 (tests/test_svd_scale_gpu.py).
 constexpr int kPjSegGroups = 32;
 
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::
-            "r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-        : "memory");
-}
-// K-major TF32 operand, 128B swizzle: rows of 32 K-contiguous floats, 8-row atoms of 1024 bytes (SBO), LBO unused
-__device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t saddr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);
-    d |= (uint64_t)1 << 16;                      // LBO (ignored for swizzled K-major layouts)
-    d |= (uint64_t)(1024 >> 4) << 32;            // SBO
-    d |= (uint64_t)1 << 46;                      // descriptor version 1 (Blackwell)
-    d |= (uint64_t)2 << 61;                      // layout type SWIZZLE_128B
-    return d;
-}
-// instruction descriptor: D fp32, A/B TF32, both K-major, M x N
-__host__ __device__ constexpr uint32_t umma_idesc_tf32_k(int M, int N) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
-// W^T planes: wt[j][tt] = tf32 split of vs[tt][col0 + j] (zero beyond r / t), [r_pad][t_pad]
-__global__ void __launch_bounds__(256)
-project_prepare_w_kernel(const float* __restrict__ vs, int64_t t, int r, int col0, int r_pad, int64_t t_pad,
-                         float* __restrict__ hi, float* __restrict__ lo) {
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= (int64_t)r_pad * t_pad) return;
-    const int j = (int)(e / t_pad);
-    const int64_t tt = e % t_pad;
-    float w = 0.f;
-    if (col0 + j < r && tt < t) w = vs[tt * r + col0 + j];
-    uint32_t hbits;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hbits) : "f"(w));
-    const float h = __uint_as_float(hbits);
-    hi[e] = h;
-    if (lo) lo[e] = w - h;
-}
-
 __global__ void __launch_bounds__(kPjThreads, 1)
 project_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo,
                   const __grid_constant__ CUtensorMap map_whi, const __grid_constant__ CUtensorMap map_wlo, int g0,
@@ -658,15 +524,10 @@ project_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
             mbar_init(&empty_bar[s], 1);
         }
         mbar_init(&acc_bar, 1);
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_hi) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_whi) : "memory");
+        tma_prefetch(&map_hi);
+        tma_prefetch(&map_whi);
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)),
-                     "r"((uint32_t)tmem_cols)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tmem_alloc(&tmem_base_slot, (uint32_t)tmem_cols);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -704,22 +565,9 @@ project_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
                 const uint32_t st = ring + (uint32_t)s * stage_bytes;
                 const uint32_t d_tmem = tmem_base + (uint32_t)((g / per_seg) * r_pad);
                 if (g % per_seg == 0) accumulate = 0;
-#pragma unroll
-                for (int ks = 0; ks < 4; ++ks) {                      // 32 floats per stage = 4 UMMA K-steps of 8
-                    const uint32_t koff = (uint32_t)ks * 32u;
-                    const uint64_t a_hi = umma_desc_k_sw128(st + koff);
-                    const uint64_t b_hi = umma_desc_k_sw128(st + 2 * kPjABytes + koff);
-                    if (passes == 3) {
-                        const uint64_t a_lo = umma_desc_k_sw128(st + kPjABytes + koff);
-                        const uint64_t b_lo = umma_desc_k_sw128(st + 2 * kPjABytes + w_bytes + koff);
-                        umma_tf32(d_tmem, a_lo, b_hi, idesc, accumulate);
-                        umma_tf32(d_tmem, a_hi, b_lo, idesc, 1u);
-                        umma_tf32(d_tmem, a_hi, b_hi, idesc, 1u);
-                    } else {
-                        umma_tf32(d_tmem, a_hi, b_hi, idesc, accumulate);
-                    }
-                    accumulate = 1u;
-                }
+                umma_stage_k(d_tmem, st, st + kPjABytes, st + 2 * kPjABytes, st + 2 * kPjABytes + w_bytes, idesc, passes,
+                             accumulate);
+                accumulate = 1u;
                 umma_commit(&empty_bar[s]);
             }
             umma_commit(&acc_bar);
@@ -754,17 +602,14 @@ project_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)tmem_cols)
-                     : "memory");
-    }
+    if (warp == 1) tmem_dealloc(tmem_base, (uint32_t)tmem_cols);
 }
 
 // ================================================================== residual of a low-rank model (s3_lowrank_error)
 //   e[m][t] = (a[m][t] - mean[m]) - sum_j left[m][j] * right_t[t][j],   j < q <= 512
 // The product runs on tcgen05 with the operand forms of project_tc_kernel: left (K = q contiguous) takes the role of the
 // planes, right_t the role of W^T; both are split into TF32 hi / lo planes ([rows_pad][q_pad], zero padded) by
-// lowrank_prepare_kernel and contracted 3xTF32 into one 128 x 256 fp32 tile in TMEM (q_pad / 8 * 3 <= 192 MMAs, one
+// tf32_split_kernel and contracted 3xTF32 into one 128 x 256 fp32 tile in TMEM (q_pad / 8 * 3 <= 192 MMAs, one
 // segment). The epilogue warps pull the tile with tcgen05.ld, read the matching 128 x 256 tile of `a` from HBM once and
 // form e in fp64. Work unit: a row tile (128 rows) over ALL column tiles, so that the row sums stay in registers of one
 // CTA; row tiles are dealt out in fixed groups of consecutive tiles (the grouping depends on m only), a group's column
@@ -783,22 +628,6 @@ constexpr int kLrTmemCols = 2 * kLrBN;
 constexpr size_t kLrSmemBytes = (size_t)kLrStages * kLrStageBytes + 1024;
 constexpr int kLrMaxGroups = 1024;                           // row-tile groups at most (scratch: groups x 3 x vol_div x t)
 int g_lowrank_cap = 0;                                       // CTAs at most (s3x_tune key 19; tests), 0 = one per SM
-
-// hi / lo TF32 planes of src [rows, q] -> [rows_pad, q_pad], zero beyond rows / q
-__global__ void __launch_bounds__(256)
-lowrank_prepare_kernel(const float* __restrict__ src, int64_t rows, int q, int64_t rows_pad, int q_pad,
-                       float* __restrict__ hi, float* __restrict__ lo) {
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= rows_pad * q_pad) return;
-    const int64_t r = e / q_pad;
-    const int j = (int)(e % q_pad);
-    const float v = (r < rows && j < q) ? src[r * q + j] : 0.f;
-    uint32_t hbits;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hbits) : "f"(v));
-    const float h = __uint_as_float(hbits);
-    hi[e] = h;
-    lo[e] = v - h;
-}
 
 // Sum over the 32 lanes of a warp of each of 32 columns, value(j) = this lane's entry of column j (reduce-scatter
 // butterfly, 31 shuffles): returns the sum (max: the maximum) of column `lane`. The order of the adds is fixed by the lane
@@ -829,8 +658,6 @@ __device__ __forceinline__ double warp_column_reduce(F value, bool max, int lane
     return v[0];
 }
 
-__device__ __forceinline__ void named_bar(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
-
 // part: fp64 [n_groups][3][vol_div][t] (sq_err, sq_ref, max_abs of the group's rows)
 __global__ void __launch_bounds__(kLrThreads, 1)
 lowrank_error_kernel(const __grid_constant__ CUtensorMap map_lhi, const __grid_constant__ CUtensorMap map_llo,
@@ -860,15 +687,10 @@ lowrank_error_kernel(const __grid_constant__ CUtensorMap map_lhi, const __grid_c
             mbar_init(&acc_full_bar[b], 1);
             mbar_init(&acc_empty_bar[b], kLrEpiWarps * 32);
         }
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_lhi) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_rhi) : "memory");
+        tma_prefetch(&map_lhi);
+        tma_prefetch(&map_rhi);
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)),
-                     "r"((uint32_t)kLrTmemCols)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tmem_alloc(&tmem_base_slot, (uint32_t)kLrTmemCols);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -915,18 +737,9 @@ lowrank_error_kernel(const __grid_constant__ CUtensorMap map_lhi, const __grid_c
                             mbar_wait_wd(&full_bar[s], (uint32_t)(it / kLrStages) & 1u);
                             tc_fence_after();
                             const uint32_t st = ring + (uint32_t)s * kLrStageBytes;
-#pragma unroll
-                            for (int ks = 0; ks < 4; ++ks) {
-                                const uint32_t koff = (uint32_t)ks * 32u;
-                                const uint64_t a_hi = umma_desc_k_sw128(st + koff);
-                                const uint64_t a_lo = umma_desc_k_sw128(st + kLrABytes + koff);
-                                const uint64_t b_hi = umma_desc_k_sw128(st + 2 * kLrABytes + koff);
-                                const uint64_t b_lo = umma_desc_k_sw128(st + 2 * kLrABytes + kLrBBytes + koff);
-                                umma_tf32(d_tmem, a_lo, b_hi, idesc, accumulate);
-                                umma_tf32(d_tmem, a_hi, b_lo, idesc, 1u);
-                                umma_tf32(d_tmem, a_hi, b_hi, idesc, 1u);
-                                accumulate = 1u;
-                            }
+                            umma_stage_k(d_tmem, st, st + kLrABytes, st + 2 * kLrABytes, st + 2 * kLrABytes + kLrBBytes,
+                                         idesc, 3, accumulate);
+                            accumulate = 1u;
                             umma_commit(&empty_bar[s]);
                         }
                         umma_commit(&acc_full_bar[b]);
@@ -1023,10 +836,7 @@ lowrank_error_kernel(const __grid_constant__ CUtensorMap map_lhi, const __grid_c
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)kLrTmemCols)
-                     : "memory");
-    }
+    if (warp == 1) tmem_dealloc(tmem_base, (uint32_t)kLrTmemCols);
 }
 
 // out[k][c][col] = sum (k = 0, 1) / max (k = 2) over the groups, in group order; part [n_groups][3][vol_div][t]
@@ -1060,10 +870,6 @@ extern "C" int s3_svd_row_means(const float* d_a, int64_t m, int64_t t, float* d
     return S3_OK;
 }
 
-typedef CUresult (*PFN_encodeTiledSvd)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                       const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                       CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 static int gram_simt(const float* d_a, const float* d_mean, const float* d_vol, int vol_div, int64_t m, int64_t t,
                      double* d_gram, cudaStream_t st) {
     const int tiles = (int)ceil_div(t, kGT);
@@ -1096,16 +902,18 @@ static int gram_simt(const float* d_a, const float* d_mean, const float* d_vol, 
     return S3_OK;
 }
 
+// Rows of A per plane chunk of gram_tc / project_tc: each plane at most 2 GB (and at most g_plane_rows_cap rows), a
+// multiple of the `tile` rows that a kernel step consumes, no more than the rows of A padded to that tile.
+static int64_t plane_rows_for(int64_t m, int64_t t_pad, int64_t tile) {
+    int64_t plane_rows = ((int64_t)(1ll << 31) / (t_pad * 4)) & ~(tile - 1);
+    if (g_plane_rows_cap > 0 && plane_rows > g_plane_rows_cap) plane_rows = g_plane_rows_cap & ~(tile - 1);
+    if (plane_rows < tile) plane_rows = tile;
+    const int64_t m_pad = ceil_div(m, tile) * tile;
+    return plane_rows < m_pad ? plane_rows : m_pad;
+}
+
 static int gram_tc(const float* d_a, const float* d_mean, const float* d_vol, int vol_div, int64_t m, int64_t t,
                    int passes, double* d_gram, cudaStream_t st) {
-    static PFN_encodeTiledSvd encode = nullptr;
-    if (!encode) {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        S3_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-        S3_REQUIRE(fn != nullptr && qres == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled not available");
-        encode = (PFN_encodeTiledSvd)fn;
-    }
     // paired kernel (clusters of two CTAs sharing B by TMA multicast): needs an even number of i-tiles per j-tile
     const bool paired = g_tc_pair != 0;
     const int64_t t_pad = paired ? ceil_div(t, kTcBN) * kTcBN : ceil_div(t, kTcBM) * kTcBM;
@@ -1115,12 +923,7 @@ static int gram_tc(const float* d_a, const float* d_mean, const float* d_vol, in
     int tiles = 0;
     if (paired) for (int tj = 0; tj < n_j; ++tj) tiles += tc_pair_count(tj, n_i);
     else for (int ti = 0; ti < n_i; ++ti) tiles += n_j - tc_first_tj(ti);
-    // rows of A per chunk: each plane at most 2 GB
-    int64_t plane_rows = ((int64_t)(1ll << 31) / (t_pad * 4)) & ~(int64_t)(kTcKB - 1);
-    if (g_plane_rows_cap > 0 && plane_rows > g_plane_rows_cap) plane_rows = g_plane_rows_cap & ~(int64_t)(kTcKB - 1);
-    if (plane_rows < kTcKB) plane_rows = kTcKB;
-    const int64_t m_pad = ceil_div(m, kTcKB) * kTcKB;
-    if (plane_rows > m_pad) plane_rows = m_pad;
+    const int64_t plane_rows = plane_rows_for(m, t_pad, kTcKB);
     int splits_max = (kNumSMs + tiles / 2) / tiles;
     if (splits_max < 1) splits_max = 1;
 
@@ -1132,22 +935,9 @@ static int gram_tc(const float* d_a, const float* d_mean, const float* d_vol, in
     S3_TRY(scratch.alloc(&partial, (size_t)tiles * splits_max * kTcBN * kTcBM));
 
     CUtensorMap map_hi, map_lo;
-    memset(&map_hi, 0, sizeof(map_hi));
-    memset(&map_lo, 0, sizeof(map_lo));
-    {
-        const cuuint64_t gdim[3] = {32, (cuuint64_t)plane_rows, (cuuint64_t)n_groups};
-        const cuuint64_t gstride[2] = {128, (cuuint64_t)plane_rows * 128};
-        const cuuint32_t box[3] = {32, (cuuint32_t)kTcKB, 4};
-        const cuuint32_t estride[3] = {1, 1, 1};
-        CUresult cr = encode(&map_hi, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, hi, gdim, gstride, box, estride,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
-                             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        S3_REQUIRE(cr == CUDA_SUCCESS, "cuTensorMapEncodeTiled(hi) failed with code %d", (int)cr);
-        cr = encode(&map_lo, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, passes == 3 ? lo : hi, gdim, gstride, box, estride,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        S3_REQUIRE(cr == CUDA_SUCCESS, "cuTensorMapEncodeTiled(lo) failed with code %d", (int)cr);
-    }
+    S3_TRY(tma_map_f32(&map_hi, "hi", hi, {32, plane_rows, n_groups}, {32, kTcKB, 4}, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B));
+    S3_TRY(tma_map_f32(&map_lo, "lo", passes == 3 ? lo : hi, {32, plane_rows, n_groups}, {32, kTcKB, 4},
+                       CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B));
     S3_CUDA(cudaFuncSetAttribute(gram_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmemBytes));
     S3_CUDA(cudaFuncSetAttribute(gram_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmemBytes));
 
@@ -1216,22 +1006,9 @@ extern "C" int s3_svd_project(const float* d_a, const float* d_mean, const float
 // U = (A - mean) vs on the tensor cores (see project_tc_kernel); vs [t, r] fp32, u [m, r] fp32.
 static int project_tc(const float* d_a, const float* d_mean, const float* d_vol, int vol_div, const float* d_vs,
                       int64_t m, int64_t t, int r, int passes, float* d_u, cudaStream_t st) {
-    static PFN_encodeTiledSvd encode = nullptr;
-    if (!encode) {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        S3_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-        S3_REQUIRE(fn != nullptr && qres == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled not available");
-        encode = (PFN_encodeTiledSvd)fn;
-    }
     const int64_t t_pad = ceil_div(t, (int64_t)32) * 32;
     const int n_groups = (int)(t_pad / 32);
-    // rows of A per chunk: each plane at most 2 GB, a multiple of the 128-row tile
-    int64_t plane_rows = ((int64_t)(1ll << 31) / (t_pad * 4)) & ~(int64_t)(kPjBM - 1);
-    if (g_plane_rows_cap > 0 && plane_rows > g_plane_rows_cap) plane_rows = g_plane_rows_cap & ~(int64_t)(kPjBM - 1);
-    if (plane_rows < kPjBM) plane_rows = kPjBM;
-    const int64_t m_pad = ceil_div(m, (int64_t)kPjBM) * kPjBM;
-    if (plane_rows > m_pad) plane_rows = m_pad;
+    const int64_t plane_rows = plane_rows_for(m, t_pad, kPjBM);
     const int r_blk_max = r < 256 ? (int)(ceil_div((int64_t)r, (int64_t)32) * 32) : 256;   // columns per pass, multiple of 32
 
     Scratch scratch(st);
@@ -1242,22 +1019,10 @@ static int project_tc(const float* d_a, const float* d_mean, const float* d_vol,
     if (passes == 3) S3_TRY(scratch.alloc(&wlo, (size_t)r_blk_max * t_pad));
 
     CUtensorMap map_hi, map_lo;
-    memset(&map_hi, 0, sizeof(map_hi));
-    memset(&map_lo, 0, sizeof(map_lo));
-    {
-        const cuuint64_t gdim[3] = {32, (cuuint64_t)plane_rows, (cuuint64_t)n_groups};
-        const cuuint64_t gstride[2] = {128, (cuuint64_t)plane_rows * 128};
-        const cuuint32_t box[3] = {32, (cuuint32_t)kPjBM, 1};
-        const cuuint32_t estride[3] = {1, 1, 1};
-        CUresult cr = encode(&map_hi, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, hi, gdim, gstride, box, estride,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        S3_REQUIRE(cr == CUDA_SUCCESS, "cuTensorMapEncodeTiled(projection hi) failed with code %d", (int)cr);
-        cr = encode(&map_lo, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, passes == 3 ? lo : hi, gdim, gstride, box, estride,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        S3_REQUIRE(cr == CUDA_SUCCESS, "cuTensorMapEncodeTiled(projection lo) failed with code %d", (int)cr);
-    }
+    S3_TRY(tma_map_f32(&map_hi, "projection hi", hi, {32, plane_rows, n_groups}, {32, kPjBM, 1},
+                       CU_TENSOR_MAP_SWIZZLE_128B));
+    S3_TRY(tma_map_f32(&map_lo, "projection lo", passes == 3 ? lo : hi, {32, plane_rows, n_groups}, {32, kPjBM, 1},
+                       CU_TENSOR_MAP_SWIZZLE_128B));
     for (int col0 = 0; col0 < r; col0 += 256) {
         const int r_blk = (r - col0) < 256 ? (r - col0) : 256;
         const int r_pad = (int)(ceil_div((int64_t)r_blk, (int64_t)32) * 32);
@@ -1267,25 +1032,13 @@ static int project_tc(const float* d_a, const float* d_mean, const float* d_vol,
         if (n_seg > 8) n_seg = 8;
         const int launch_groups = n_seg * kPjSegGroups;            // t range of one launch: segments of <= kPjSegGroups
         if (n_seg > n_groups) n_seg = n_groups;
-        project_prepare_w_kernel<<<(unsigned)ceil_div((int64_t)r_pad * t_pad, (int64_t)256), 256, 0, st>>>(
-            d_vs, t, r, col0, r_pad, t_pad, whi, wlo);
+        // W^T [r_pad][t_pad]: W^T[j][tt] = vs[tt][col0 + j]
+        tf32_split_kernel<<<(unsigned)ceil_div((int64_t)r_pad * t_pad, (int64_t)256), 256, 0, st>>>(
+            d_vs + col0, 1, r, r_blk, t, r_pad, t_pad, whi, wlo);
         CUtensorMap map_whi, map_wlo;
-        memset(&map_whi, 0, sizeof(map_whi));
-        memset(&map_wlo, 0, sizeof(map_wlo));
-        {
-            const cuuint64_t gdim[2] = {(cuuint64_t)t_pad, (cuuint64_t)r_pad};
-            const cuuint64_t gstride[1] = {(cuuint64_t)t_pad * 4};
-            const cuuint32_t box[2] = {32, (cuuint32_t)r_pad};
-            const cuuint32_t estride[2] = {1, 1};
-            CUresult cr = encode(&map_whi, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, whi, gdim, gstride, box, estride,
-                                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            S3_REQUIRE(cr == CUDA_SUCCESS, "cuTensorMapEncodeTiled(projection W hi) failed with code %d", (int)cr);
-            cr = encode(&map_wlo, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, passes == 3 ? wlo : whi, gdim, gstride, box, estride,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            S3_REQUIRE(cr == CUDA_SUCCESS, "cuTensorMapEncodeTiled(projection W lo) failed with code %d", (int)cr);
-        }
+        S3_TRY(tma_map_f32(&map_whi, "projection W hi", whi, {t_pad, r_pad}, {32, r_pad}, CU_TENSOR_MAP_SWIZZLE_128B));
+        S3_TRY(tma_map_f32(&map_wlo, "projection W lo", passes == 3 ? wlo : whi, {t_pad, r_pad}, {32, r_pad},
+                           CU_TENSOR_MAP_SWIZZLE_128B));
         const size_t smem = (size_t)kPjStages * (2 * kPjABytes + 2 * (size_t)r_pad * 128) + 1024;
         S3_CUDA(cudaFuncSetAttribute(project_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         for (int64_t row0 = 0; row0 < m; row0 += plane_rows) {
@@ -1335,14 +1088,6 @@ extern "C" int s3_lowrank_error(const float* d_a, int64_t m, int64_t t, const fl
         return S3_ERR_UNSUPPORTED;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    static PFN_encodeTiledSvd encode = nullptr;
-    if (!encode) {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        S3_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-        S3_REQUIRE(fn != nullptr && qres == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled not available");
-        encode = (PFN_encodeTiledSvd)fn;
-    }
     const int q_pad = (int)(ceil_div((int64_t)q, (int64_t)32) * 32);
     const int64_t m_pad = ceil_div(m, (int64_t)kLrBM) * kLrBM, t_pad = ceil_div(t, (int64_t)kLrBN) * kLrBN;
     const int64_t n_rt = m_pad / kLrBM;
@@ -1361,23 +1106,15 @@ extern "C" int s3_lowrank_error(const float* d_a, int64_t m, int64_t t, const fl
     S3_TRY(scratch.alloc(&rhi, (size_t)t_pad * q_pad));
     S3_TRY(scratch.alloc(&rlo, (size_t)t_pad * q_pad));
     S3_TRY(scratch.alloc(&part, (size_t)n_groups * 3 * vol_div * t));
-    lowrank_prepare_kernel<<<(unsigned)ceil_div(m_pad * q_pad, (int64_t)256), 256, 0, st>>>(d_left, m, q, m_pad, q_pad,
-                                                                                          lhi, llo);
-    lowrank_prepare_kernel<<<(unsigned)ceil_div(t_pad * q_pad, (int64_t)256), 256, 0, st>>>(d_right_t, t, q, t_pad,
-                                                                                          q_pad, rhi, rlo);
+    tf32_split_kernel<<<(unsigned)ceil_div(m_pad * q_pad, (int64_t)256), 256, 0, st>>>(d_left, q, 1, m, q, m_pad, q_pad,
+                                                                                     lhi, llo);
+    tf32_split_kernel<<<(unsigned)ceil_div(t_pad * q_pad, (int64_t)256), 256, 0, st>>>(d_right_t, q, 1, t, q, t_pad,
+                                                                                     q_pad, rhi, rlo);
     CUtensorMap maps[4];
-    float* planes[4] = {lhi, llo, rhi, rlo};
-    for (int i = 0; i < 4; ++i) {
-        memset(&maps[i], 0, sizeof(CUtensorMap));
-        const cuuint64_t gdim[2] = {(cuuint64_t)q_pad, (cuuint64_t)(i < 2 ? m_pad : t_pad)};
-        const cuuint64_t gstride[1] = {(cuuint64_t)q_pad * 4};
-        const cuuint32_t box[2] = {32, (cuuint32_t)(i < 2 ? kLrBM : kLrBN)};
-        const cuuint32_t estride[2] = {1, 1};
-        CUresult cr = encode(&maps[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, planes[i], gdim, gstride, box, estride,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        S3_REQUIRE(cr == CUDA_SUCCESS, "cuTensorMapEncodeTiled(low-rank plane %d) failed with code %d", i, (int)cr);
-    }
+    S3_TRY(tma_map_f32(&maps[0], "low-rank left hi", lhi, {q_pad, m_pad}, {32, kLrBM}, CU_TENSOR_MAP_SWIZZLE_128B));
+    S3_TRY(tma_map_f32(&maps[1], "low-rank left lo", llo, {q_pad, m_pad}, {32, kLrBM}, CU_TENSOR_MAP_SWIZZLE_128B));
+    S3_TRY(tma_map_f32(&maps[2], "low-rank right hi", rhi, {q_pad, t_pad}, {32, kLrBN}, CU_TENSOR_MAP_SWIZZLE_128B));
+    S3_TRY(tma_map_f32(&maps[3], "low-rank right lo", rlo, {q_pad, t_pad}, {32, kLrBN}, CU_TENSOR_MAP_SWIZZLE_128B));
     S3_CUDA(cudaFuncSetAttribute(lowrank_error_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrSmemBytes));
     lowrank_error_kernel<<<(unsigned)ctas, kLrThreads, kLrSmemBytes, st>>>(
         maps[0], maps[1], maps[2], maps[3], d_a, d_mean, d_vol, vol_div, m, t, q_pad / 32, n_ct, n_rt, tiles_per_group,

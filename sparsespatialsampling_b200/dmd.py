@@ -101,8 +101,7 @@ def compute_dmd(data_matrix: pt.Tensor, cell_area: pt.Tensor, dt: float, rank: i
         its results back): ``DMD.reconstruction_error`` contracts the modes there, and ``.cpu()`` is one call away
     """
     _lib.require_cuda()
-    if method not in svd.GRAM_METHODS:
-        raise ValueError(f"unknown Gram method '{method}', available: {sorted(svd.GRAM_METHODS)}")
+    svd._check_method(method)
     shape = tuple(data_matrix.shape)
     if len(shape) not in (2, 3):
         raise ValueError(f"data_matrix must be [N_cells, T] or [N_cells, D, T], got {shape}")
@@ -115,11 +114,7 @@ def compute_dmd(data_matrix: pt.Tensor, cell_area: pt.Tensor, dt: float, rank: i
     zero = pt.zeros((a.size(0),), dtype=pt.float32, device=dev)
 
     g = svd.gram(a, zero, vol, vol_div, method)
-    g1 = g[:-1, :-1]
-    r_max = min(a.size(0), t - 1)
-    lam, vec = svd.eigenpairs(g1, rank, r_max)
-    s_all = lam.clamp_min(0.0).sqrt()
-    r = svd.optimal_rank(s_all[:r_max], a.size(0), t - 1) if rank is None else max(1, min(int(rank), r_max))
+    s_all, vec, r = svd._spectrum(g[:-1, :-1], rank, a.size(0), t - 1)
     # the cutoff of compute_svd's modes: below 1e-6 sigma_0, S^-1 only amplifies the rounding of G (whose 1e-6 accuracy
     # holds for sigma^2, so singular values below about 1e-3 sigma_0 that are kept already carry that rounding)
     live = int((s_all[:r] > 1e-6 * float(s_all[0])).sum()) if float(s_all[0]) > 0 else 0
@@ -147,7 +142,7 @@ def compute_dmd(data_matrix: pt.Tensor, cell_area: pt.Tensor, dt: float, rank: i
     coef = pt.zeros((t, 2 * n), dtype=pt.float32, device=dev)              # row 0: X[:, 0] is not in X[:, 1:]
     coef[1:, :n] = c[:, :n].real.float()
     coef[1:, n:] = c[:, :n].imag.float()
-    u = svd.project(a, zero, coef) if method == "simt" else svd.project_tc(a, zero, vol, vol_div, coef, method)
+    u = svd._project(a, zero, vol, vol_div, coef, method)
     modes = pt.complex(u[:, :n], u[:, n:])
     modes = modes.reshape(shape[:-1] + (n,))
     return DMD(s, eigvals, amplitude, modes, dt, t, vol, shape)

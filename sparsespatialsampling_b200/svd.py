@@ -33,6 +33,11 @@ logger = logging.getLogger(__name__)
 GRAM_METHODS = {"simt": 0, "tc3": 1, "tc": 2}
 
 
+def _check_method(method: str):
+    if method not in GRAM_METHODS:
+        raise ValueError(f"unknown Gram method '{method}', available: {sorted(GRAM_METHODS)}")
+
+
 def optimal_rank(s: pt.Tensor, rows: int, cols: int) -> int:
     """Optimal hard threshold for singular values, unknown noise level (Gavish & Donoho 2014, eq. 5):
     rank = #{s_i > omega(beta) * median(s)}, omega(beta) ~ 0.56 b^3 - 0.95 b^2 + 1.82 b + 1.43, beta = min/max."""
@@ -114,6 +119,11 @@ def project_tc(a: pt.Tensor, mean: pt.Tensor, vol: pt.Tensor, vol_div: int, vs: 
         _lib.check(lib.s3_svd_project_tc(_lib.ptr(a), _lib.ptr(mean), _lib.ptr(vol), vol_div, _lib.ptr(vs), a.size(0),
                                          a.size(1), vs.size(1), GRAM_METHODS[method], _lib.ptr(u), _lib.stream_ptr()))
     return u
+
+
+def _project(a: pt.Tensor, mean: pt.Tensor, vol: pt.Tensor, vol_div: int, vs: pt.Tensor, method: str) -> pt.Tensor:
+    """``(a - mean[:, None]) @ vs`` by the projection kernel that goes with the Gram ``method``."""
+    return project(a, mean, vs) if method == "simt" else project_tc(a, mean, vol, vol_div, vs, method)
 
 
 LOWRANK_MAX_Q = 512
@@ -209,18 +219,15 @@ def compute_svd(data_matrix: pt.Tensor, cell_area: pt.Tensor, rank: int = None, 
     :return: ``(s [r], U [N_cells, r] | [N_cells, D, r], V [T, r])`` on the device of ``data_matrix``
     """
     _lib.require_cuda()
-    if method not in GRAM_METHODS:
-        raise ValueError(f"unknown Gram method '{method}', available: {sorted(GRAM_METHODS)}")
+    _check_method(method)
     shape = tuple(data_matrix.shape)
     home = data_matrix.device
     a, vol, vol_div, dev = _field_on_device(data_matrix, cell_area, device)
-    n_cells = shape[0]
 
     mean = row_means(a)
     g = gram(a, mean, vol, vol_div, method)
     s_out, u, v_out = _factor(a, mean, g, rank, n_modes, a.size(0), vol, vol_div, method)
-    if len(shape) == 3:
-        u = u.reshape(n_cells, vol_div, u.size(-1))
+    u = u.reshape(shape[:-1] + (u.size(-1),))
     if home != dev:
         pt.cuda.synchronize(dev)
         return s_out.to(home), u.to(home), v_out.to(home)
@@ -306,25 +313,27 @@ def eigenpairs(g: pt.Tensor, rank, r_max: int):
     return pt.flip(lam, dims=(0,)), pt.flip(vec, dims=(1,))
 
 
+def _spectrum(g: pt.Tensor, rank, rows: int, cols: int):
+    """``(s_all, vec, r)``: singular values (descending) and right singular vectors of a ``rows x cols`` matrix from its
+    Gram matrix ``g``; ``r`` = ``rank`` clamped to ``[1, min(rows, cols)]``, or the optimal hard threshold for ``None``."""
+    r_max = min(rows, cols)
+    lam, vec = eigenpairs(g, rank, r_max)
+    s_all = lam.clamp_min(0.0).sqrt()
+    r = optimal_rank(s_all[:r_max], rows, cols) if rank is None else max(1, min(int(rank), r_max))
+    return s_all, vec, r
+
+
 def _factor(a: pt.Tensor, mean: pt.Tensor, g: pt.Tensor, rank, n_modes, rows_total: int, vol: pt.Tensor, vol_div: int,
             method: str):
     """Eigen-decomposition of the (summed) Gram matrix and projection of the rows held in ``a``."""
-    t = a.size(1)
-    r_max = min(rows_total, t)
-    lam, vec = eigenpairs(g, rank, r_max)
-    s_all = lam.clamp_min(0.0).sqrt()
-    if rank is None:
-        r = optimal_rank(s_all[:r_max], rows_total, t)
-    else:
-        r = max(1, min(int(rank), r_max))
+    s_all, vec, r = _spectrum(g, rank, rows_total, a.size(1))
     s = s_all[:r]
     v = vec[:, :r]
     r_u = r if n_modes is None else max(1, min(int(n_modes), r))
     live = s[:r_u] > 1e-6 * float(s_all[0]) if float(s_all[0]) > 0 else pt.zeros(r_u, dtype=pt.bool, device=a.device)
     inv_s = pt.where(live, 1.0 / s[:r_u].clamp_min(1e-300), pt.zeros_like(s[:r_u]))
     vs = v[:, :r_u] * inv_s.unsqueeze(0)
-    u = project(a, mean, vs) if method == "simt" else project_tc(a, mean, vol, vol_div, vs, method)
-    return s.to(pt.float32), u, v.to(pt.float32)
+    return s.to(pt.float32), _project(a, mean, vol, vol_div, vs, method), v.to(pt.float32)
 
 
 def compute_svd_sharded(data_local: pt.Tensor, cell_area_local: pt.Tensor, rank: int = None, method: str = "tc3",
@@ -347,8 +356,7 @@ def compute_svd_sharded(data_local: pt.Tensor, cell_area_local: pt.Tensor, rank:
     """
     from . import parallel
     _lib.require_cuda()
-    if method not in GRAM_METHODS:
-        raise ValueError(f"unknown Gram method '{method}', available: {sorted(GRAM_METHODS)}")
+    _check_method(method)
     if sharded_by not in ("cells", "time"):
         raise ValueError(f"sharded_by must be 'cells' or 'time', got '{sharded_by}'")
     if data_local.device.type != "cuda":
@@ -366,15 +374,7 @@ def compute_svd_sharded(data_local: pt.Tensor, cell_area_local: pt.Tensor, rank:
             import torch.distributed as dist
             r0, r1 = parallel.row_window(n_cells_total, dist.get_world_size(group), dist.get_rank(group))
             area = area[r0:r1]
-    shape = tuple(data_local.shape)
-    if len(shape) not in (2, 3):
-        raise ValueError(f"data_local must be [n, T] or [n, D, T], got {shape}")
-    if area.numel() != shape[0]:
-        raise ValueError(f"cell_area has {area.numel()} entries for {shape[0]} local cells")
-    n_local, t = shape[0], shape[-1]
-    vol_div = 1 if len(shape) == 2 else shape[1]
-    a = _as_device_matrix(data_local, dev).reshape(n_local * vol_div, t)
-    vol = area.to(device=dev, dtype=pt.float32).contiguous()
+    a, vol, vol_div, _ = _field_on_device(data_local, area, dev)
 
     mean = row_means(a)
     g = gram(a, mean, vol, vol_div, method)
@@ -383,8 +383,7 @@ def compute_svd_sharded(data_local: pt.Tensor, cell_area_local: pt.Tensor, rank:
     parallel.allreduce_sum(counts, group)
     rows_total = int(counts.item())
     s_out, u, v_out = _factor(a, mean, g, rank, n_modes, rows_total, vol, vol_div, method)
-    if len(shape) == 3:
-        u = u.reshape(n_local, vol_div, u.size(-1))
+    u = u.reshape(data_local.shape[:-1] + (u.size(-1),))
     if gather_modes:
         u = parallel.gather_rows(u, rows_total // vol_div, group)
     return s_out, u, v_out
