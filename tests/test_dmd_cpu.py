@@ -68,6 +68,21 @@ def test_gram_algebra_matches_the_oracle(host, d):
     assert np.allclose(dmd.dynamics.numpy()[:, 5], dmd.amplitude.numpy() * dmd.eigvals.numpy() ** 5, rtol=1e-10)
 
 
+@pytest.mark.parametrize("d,rank", [(None, 6), (3, 20)])
+def test_torch_oracle_matches_the_numpy_oracle(d, rank):
+    """The fp64 torch port (QR of the weighted X1, the reference of the GPU tests at production sizes) against the
+    numpy oracle (SVD of the weighted X1), rank beyond the six signal pairs included, ``block`` smaller than M."""
+    a, area, _ = _oscillations(400, 60, d, noise=1e-3, seed=4)
+    lam, b, phi, s = dmd_oracle.compute_dmd(a, area, rank)
+    lam_t, b_t, phi_t, s_t = dmd_oracle.compute_dmd_torch(pt.from_numpy(a), pt.from_numpy(area), rank, block=128)
+    assert tuple(phi_t.shape) == phi.shape and phi_t.dtype == pt.complex128
+    assert np.abs(s_t.numpy() - s[:rank]).max() <= 1e-12 * s[0]
+    assert np.abs(lam_t.numpy() - lam).max() <= 1e-9
+    got = phi_t.numpy() * b_t.numpy()
+    want = phi * b
+    assert np.abs(got - want).max() <= 1e-9 * np.abs(want).max()
+
+
 def test_n_modes_and_rank_clamps(host, caplog):
     from sparsespatialsampling_b200.dmd import compute_dmd
     a, area, dt = _oscillations(200, 12, seed=2)
